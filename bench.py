@@ -6,6 +6,8 @@ warp HBM GB/s).
     python bench.py --config seg|reg|warp-sweep|batch64 ...             # BASELINE configs[0], [1], [4], [3]
     python bench.py --impl reference --gpus 1 --steps 2 --warmup 1      # the reference's CPU path (oracle port)
     torchrun ... bench.py --gpus N ...                                  # N ranks, knees sharded by volume, no collective
+    python bench.py --steps 5 --warmup 3 --dump-outputs DIR             # --config full only: also write the last
+                                                                        # timed step's outputs to DIR/<name>.npy
 
 --config full (default): one "step" = one synthetic 160x384x384 knee through 3-D UNet segmentation (160 overlapping
 32x128x128 tiles), GradICON registration to the atlas (both directions), warp of the FC/TC probability maps onto the
@@ -169,6 +171,23 @@ def make_inputs(rank, n_distinct=2):
     return vols, verts
 
 
+DUMP_BYTES_PER_ARRAY = 8 << 20   # the five outputs of --config full stay under 64 MB in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each output as <out_dir>/<name>.npy in its own dtype (float32 / float64).  An array larger than
+    DUMP_BYTES_PER_ARRAY is written as a sample of its flattened elements at sorted indices drawn with a fixed seed, so
+    two builds run with the same arguments can be compared value for value."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        k = DUMP_BYTES_PER_ARRAY // a.itemsize
+        if a.size > k:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def conv_profile_end(lib, check):
     ms, n, fl, xfl = ctypes.c_double(), ctypes.c_longlong(), ctypes.c_double(), ctypes.c_double()
     check(lib.oai_profile_end(ctypes.byref(ms), ctypes.byref(n), ctypes.byref(fl), ctypes.byref(xfl)), "profile")
@@ -286,7 +305,7 @@ def run_full(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        step_device(i)
+        last = step_device(i)
     e1.record()
     torch.cuda.synchronize()
     conv_ms, conv_n, conv_fl, conv_xfl = conv_profile_end(_lib.lib, _lib.check)
@@ -301,6 +320,10 @@ def run_full(args):
     ms = sharding.max_over_ranks(e0.elapsed_time(e1), world)
     ms_per_step = ms / args.steps
     value = world * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # before the e2e arm below replays the graph, which overwrites the static outputs `last` aliases
+        dump_outputs(args.dump_outputs, dict(prob=last["prob"], warped=last["warped"], phi_AB=last["phi_AB"].disp,
+                                             phi_BA=last["phi_BA"].disp, vertices=last["vertices"]))
 
     # end to end through the public host API: pinned host volume in, atlas-space maps / fields / vertices out
     pipe.run(vols_pin[0], geom, verts_pin)  # allocates the pinned result buffers
@@ -935,7 +958,15 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying the CUDA graph")
     ap.add_argument("--overlap-registration", action="store_true",
                     help="A/B: record the registration as a parallel branch of the per-knee graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--config full: write what the last timed step computed (rank 0) to DIR/<name>.npy: the FC/TC "
+                         "probability maps (prob), the maps on the atlas grid (warped), the displacement fields of both "
+                         "directions (phi_AB, phi_BA) and the warped vertices; arrays over 8 MB as a fixed-seed sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "full"):
+        ap.error("--dump-outputs is implemented for --impl b200 --config full")
     if args.precision:
         os.environ["OAI_B200_SEG_PRECISION"] = args.precision
     if args.impl == "reference":

@@ -1,17 +1,17 @@
 """CPU tier: UNet.weights_init (SURVEY row a6; reference oai_analysis/segmentation/networks.py:71-78, reached through
 initialize_model(ckpoint_path=None), utils.py:42-44): xavier_normal_ on every conv weight, zero bias, BatchNorm left at
-its defaults -- checked statistically, and draw for draw against the reference's own module when /root/reference is
-present (build container only)."""
+its defaults -- checked statistically, and draw for draw against the reference's nn.Module restated below."""
 import math
-import os
-import sys
 
 import numpy as np
 import pytest
 import torch
+from torch import nn
 
+from helpers import load_golden
 from oai_analysis_2_b200.segmentation.networks import UNet
 from oai_analysis_2_b200.segmentation.utils import initialize_model
+from oracle.seg_oracle import make_unet_state_dict
 
 
 def test_weights_init_statistics():
@@ -46,14 +46,53 @@ def test_weights_init_invalidates_packed_handles_and_keeps_keys():
     assert net._handles == {} and set(net.state_dict()) == keys
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/oai_analysis"), reason="reference sources not on this box")
+class RefUNet(nn.Module):
+    """The reference UNet as an nn.Module (networks.py:39-66 constructor, encoder/decoder blocks :80-107, weights_init
+    :71-78): submodules registered in the reference's order -- ec0..ec7 at :43-50, pool0..2 at :52-54, dc9..dc1 at
+    :56-64, dc0 at :66 (SURVEY §2.2 and row a4) -- so self.modules() visits the conv layers, and weights_init draws, in
+    the order the reference does.  Its state-dict keys and shapes are pinned to the reference's own by
+    test_reference_module_takes_the_golden_fixture_state_dicts.  forward() is not needed here."""
+
+    def __init__(self, in_channel, n_classes, bias=False, BN=False):
+        super().__init__()
+        for name, ci, co in (("ec0", in_channel, 32), ("ec1", 32, 64), ("ec2", 64, 64), ("ec3", 64, 128),
+                             ("ec4", 128, 128), ("ec5", 128, 256), ("ec6", 256, 256), ("ec7", 256, 512)):
+            setattr(self, name, self.block(nn.Conv3d(ci, co, 3, stride=1, padding=1, bias=bias), co, BN))
+        self.pool0, self.pool1, self.pool2 = nn.MaxPool3d(2), nn.MaxPool3d(2), nn.MaxPool3d(2)
+        for name, ci, co, k, s, p in (("dc9", 512, 512, 2, 2, 0), ("dc8", 256 + 512, 256, 3, 1, 1),
+                                      ("dc7", 256, 256, 3, 1, 1), ("dc6", 256, 256, 2, 2, 0),
+                                      ("dc5", 128 + 256, 128, 3, 1, 1), ("dc4", 128, 128, 3, 1, 1),
+                                      ("dc3", 128, 128, 2, 2, 0), ("dc2", 64 + 128, 64, 3, 1, 1),
+                                      ("dc1", 64, 64, 3, 1, 1)):
+            setattr(self, name, self.block(nn.ConvTranspose3d(ci, co, k, stride=s, padding=p, bias=bias), co, BN))
+        self.dc0 = nn.Conv3d(64, n_classes, 1, bias=bias)
+
+    @staticmethod
+    def block(conv, co, BN):
+        return nn.Sequential(conv, nn.BatchNorm3d(co), nn.ReLU()) if BN else nn.Sequential(conv, nn.ReLU())
+
+    def weights_init(self):
+        for m in self.modules():
+            if "Conv" in m.__class__.__name__:
+                nn.init.xavier_normal_(m.weight.data)
+                if m.bias is not None:
+                    m.bias.data.zero_()
+
+
+@pytest.mark.parametrize("name", ["seg_small_pertap", "seg_small_nobn"])
+def test_reference_module_takes_the_golden_fixture_state_dicts(name):
+    """The reference's own checkpoint loader (utils.py:20-41, strict) loaded exactly these state dicts into its UNet to
+    produce tests/golden/<name>.npz (make_golden.py), so they carry the reference's keys and shapes: every transposed
+    conv's [cin, cout, k, k, k] layout, dc0 as a 1x1x1 conv with its bias.  The restatement must take them the same
+    way (a missing / unexpected key or a shape mismatch raises)."""
+    _, m = load_golden(name)
+    sd = make_unet_state_dict(m["seed"], 1, 2, m["bias"], m["BN"], True, m["head_gain"], m["head_bias"])
+    ref = RefUNet(1, 2, bias=m["bias"], BN=m["BN"])
+    ref.load_state_dict(sd, strict=True)
+
+
 def test_weights_init_draws_match_the_reference_module():
     """Same seed, same draw order: the state dict equals the reference UNet's after its own weights_init()."""
-    sys.path.insert(0, "/root/reference")
-    try:
-        from oai_analysis.segmentation.networks import UNet as RefUNet
-    finally:
-        sys.path.remove("/root/reference")
     torch.manual_seed(1234)
     ref = RefUNet(1, 2, bias=True, BN=True)
     torch.manual_seed(99)
