@@ -351,6 +351,36 @@ OAI_API int oai_reg_field(oai_reg_t handle, int index, size_t* workspace_offset,
 OAI_API int oai_reg_warp_image(oai_reg_t handle, const float* image, const int* dims, int direction, float* out,
                                void* workspace, size_t workspace_bytes, void* stream);
 
+/* Registration quality: the terms of icon_registration's GradientICON.forward(A, B), i.e. its ICONLoss tuple, for the
+ * last pair oai_reg_forward registered on reg_workspace (read only; nothing is written into it).  At the network shape:
+ *   similarity          = sim(S(A, phi_AB), B) + sim(S(B, phi_BA), A) on the resized pair, sim = LNCC(sigma) (Gaussian
+ *                         of 2*floor(2*sigma)+1 taps, zero padding) or ssd_only_interpolated (in-bounds tag warped
+ *                         with the image);
+ *   inverse consistency = sum_d mean(((e(Ie) - e(Ie + delta*e_d)) / delta)^2), e(c) = c - phi_AB(phi_BA(c)),
+ *                         Ie = identity + noise / W, noise: device float32 [3][net_dims] of N(0, 1) values;
+ *   transform magnitude = mean((identity - phi_AB)^2);  flips = #{dV < 0} of phi_BA (losses.flips);
+ *   all                 = lmbda * inverse consistency + similarity.
+ * terms: device double[5] in ICONLoss order (all, inverse consistency, similarity, transform magnitude, flips).
+ * jac_det_BA (optional): device float32 [D-1][H-1][W-1], the dV map of phi_BA.  loss_workspace: 256-byte aligned
+ * device memory of oai_reg_loss_workspace_bytes(handle, cfg) bytes (oai_reg_workspace_bytes is unaffected).
+ * Fixed-order reductions (equal inputs give bitwise equal terms); no host synchronisation, no allocation. */
+#define OAI_SIM_LNCC 0
+#define OAI_SIM_SSD_ONLY_INTERPOLATED 1
+typedef struct {
+  int similarity;   /* OAI_SIM_LNCC or OAI_SIM_SSD_ONLY_INTERPOLATED */
+  double sigma;     /* LNCC Gaussian sigma in voxels, 0 < sigma < 12.5 (ignored by ssd_only_interpolated) */
+  double lmbda;     /* weight of the inverse-consistency term in `all` */
+  double delta;     /* finite-difference step of the gradient-ICON term (icon: 1e-3) */
+} oai_icon_loss_cfg;
+OAI_API size_t oai_reg_loss_workspace_bytes(oai_reg_t handle, const oai_icon_loss_cfg* cfg);
+OAI_API int oai_reg_icon_loss(oai_reg_t handle, const oai_icon_loss_cfg* cfg, const float* noise, double* terms,
+                              float* jac_det_BA, void* loss_workspace, size_t loss_workspace_bytes,
+                              const void* reg_workspace, size_t reg_workspace_bytes, void* stream);
+/* losses.flips on any map phi: device float32 [3][dims] (z,y,x channels): dV = ((a x b) . c) with forward differences
+ * a, b, c along z, y, x at cells [1:, 1:, 1:]; *count_out (device int64) = #{dV < 0}, exact; det_out (optional) =
+ * device float32 [D-1][H-1][W-1].  Every axis needs at least 2 samples. */
+OAI_API int oai_jacobian_flips(const float* phi, const int* dims, float* det_out, long long* count_out, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------------
  * ITK-semantics warps  (reference: oai_analysis/dask_processing.py:95-111 deform_probmap_delayed,
  * test/test_all.py:42-52; transform = R_A o DisplacementFieldTransform o R_B^-1 built by create_itk_transform)

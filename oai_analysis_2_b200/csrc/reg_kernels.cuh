@@ -119,4 +119,61 @@ int disp_field_launch(const float* phi, int D, int H, int W, float* disp, cudaSt
 int warp_volume_launch(const WarpVolumeParams& p, cudaStream_t st);
 int warp_points_launch(const WarpPointsParams& p, cudaStream_t st);
 
+// ---- registration-quality terms of GradientICON.forward (reg_loss.cu)
+struct GradIconParams {
+  int D, H, W;               // grid of the noisy identity map Ie = identity + noise / W
+  const float* noise;        // [3][D][H][W] N(0, 1)
+  float delta;               // finite-difference step along each coordinate channel
+  int nf[2];                 // fields of the two maps: [0] applied first (phi_BA), [1] then (phi_AB)
+  const float* u[2][4];      // [3][ud][uh][uw] displacement fields in application order
+  int ud[2][4], uh[2][4], uw[2][4];
+  double* partials;          // [gradicon_blocks]
+};
+
+struct JacobianParams {
+  int D, H, W;
+  const float* phi_jac;      // [3][D][H][W] map whose dV / folds are counted
+  const float* phi_mag;      // optional [3][D][H][W] map of mean((identity - phi)^2)
+  float* det_out;            // optional dV map [D-1][H-1][W-1]
+  unsigned long long* count; // device counter of dV < 0 (reset by jacobian_launch)
+  double* mag_partials;      // [jacobian_blocks] when phi_mag is set
+};
+
+constexpr int kLnccMaxRadius = 24;   // taps 2R + 1 with R = floor(2 sigma): sigma < 12.5
+struct LnccParams {
+  int D, H, W;
+  const float* I;            // warped image
+  const float* J;            // target
+  int radius;
+  float taps[2 * kLnccMaxRadius + 1];   // normalised Gaussian, 2 * radius + 1 used
+  float* zb;                 // scratch [5][D][H][W]: the moments blurred along z
+  double* partials;          // [lncc_blocks]: sums of 1 - NCC
+};
+
+struct LossFinishParams {
+  const double* g;           // gradicon partials
+  int ng;
+  const double* s;           // similarity partials [2 directions][2][ns]: LNCC uses [d][0]; SSD numerator, divisor
+  int ns, ssd;
+  const double* m;           // transform-magnitude partials
+  int nm;
+  const unsigned long long* count;
+  double nvox, lmbda;
+  double* terms;             // ICONLoss order: all, inverse consistency, similarity, transform magnitude, flips
+};
+
+int gradicon_blocks(int D, int H, int W);
+int jacobian_blocks(int D, int H, int W);
+int lncc_blocks(int D, int H, int W);
+int ssd_blocks(int D, int H, int W);
+int lncc_radius(double sigma);
+size_t lncc_tile_smem(int radius);
+int gradicon_launch(const GradIconParams& p, cudaStream_t st);
+int jacobian_launch(const JacobianParams& p, cudaStream_t st);
+int lncc_launch(const LnccParams& p, cudaStream_t st);
+int ssd_launch(const float* warped, const float* tag, const float* target, int D, int H, int W, double* num,
+               double* den, cudaStream_t st);
+int inbounds_tag_launch(float* tag, int D, int H, int W, cudaStream_t st);
+int loss_finish_launch(const LossFinishParams& p, cudaStream_t st);
+
 }  // namespace oai

@@ -282,6 +282,7 @@ struct Ctx {
   size_t scratch_need = 0;
   std::map<std::array<int, 3>, Geo> geos;
   std::vector<FieldRef> fields;   // every leaf's displacement field, evaluation order
+  size_t pair_off = 0;            // arena offset of the resized pair [A, B] (Slots::src)
 
   void* alloc(size_t bytes) {
     off = align256(off);
@@ -320,6 +321,8 @@ struct oai_reg_handle {
   std::string description;
   size_t scratch_bytes = 0, arena_bytes = 0;
   std::vector<FieldRef> fields;       // application order of the whole cascade (first applied first)
+  size_t pair_off = 0;                // arena offset of the resized pair [A, B] at the network shape
+  bool forwarded = false;             // oai_reg_forward has run at least once (the loss reads its results)
 };
 
 namespace {
@@ -493,6 +496,7 @@ int run(Ctx& c, const float* A, const int* dims_A, const float* B, const int* di
   s.src = static_cast<float*>(c.alloc(sizeof(float) * kBatch * vol));
   s.tgt = static_cast<float*>(c.alloc(sizeof(float) * kBatch * vol));
   s.phi = static_cast<float*>(c.alloc(sizeof(float) * kBatch * 3 * vol));
+  c.pair_off = static_cast<size_t>(reinterpret_cast<char*>(s.src) - c.arena);
   if (!c.dry) {   // itk_wrapper.register_pair: F.interpolate(size=shape, mode="trilinear", align_corners=False)
     RC(resize_trilinear_launch(A, dims_A[0], dims_A[1], dims_A[2], s.src, dims[0], dims[1], dims[2], c.st));
     RC(resize_trilinear_launch(B, dims_B[0], dims_B[1], dims_B[2], s.src + vol, dims[0], dims[1], dims[2], c.st));
@@ -642,6 +646,7 @@ extern "C" int oai_reg_create(const oai_tensor* state_dict, int n_tensors, const
     return bail(rc);
   h->scratch_bytes = align256(std::max<size_t>(c.scratch_need, 256));
   h->arena_bytes = align256(c.off);
+  h->pair_off = c.pair_off;
   *handle = h;
   return 0;
 }
@@ -698,6 +703,7 @@ extern "C" int oai_reg_forward(oai_reg_t h, const float* image_A, const int* dim
   if (rc) return rc;
   OAI_REQUIRE(align256(c.off) == h->arena_bytes && c.scratch_need <= h->scratch_bytes,
               "reg_forward: workspace plan mismatch (%zu vs %zu bytes)", align256(c.off), h->arena_bytes);
+  h->forwarded = true;
   return 0;
 }
 
@@ -716,4 +722,176 @@ extern "C" int oai_reg_warp_image(oai_reg_t h, const float* image, const int* di
     fields.push_back(f);
   }
   return compose(c, fields, direction, dims, image, dims, nullptr, out);
+}
+
+// ---- registration quality (GradientICON.forward's ICONLoss terms) on the last forward's workspace
+namespace {
+
+struct LossPlan {
+  size_t phi, warped, tag, wtag, zb, g, s, m, count, total;   // byte offsets inside the loss workspace
+  int ng, ns, nm;
+};
+
+LossPlan loss_plan(const oai_reg_handle* h, const oai_icon_loss_cfg& cfg) {
+  const int D = h->dims[0], H = h->dims[1], W = h->dims[2];
+  const size_t vol = voxels(h->dims);
+  const bool ssd = cfg.similarity == OAI_SIM_SSD_ONLY_INTERPOLATED;
+  LossPlan p{};
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    const size_t at = align256(off);
+    off = at + bytes;
+    return at;
+  };
+  p.ng = gradicon_blocks(D, H, W);
+  p.ns = ssd ? ssd_blocks(D, H, W) : lncc_blocks(D, H, W);
+  p.nm = jacobian_blocks(D, H, W);
+  p.phi = take(sizeof(float) * kBatch * 3 * vol);    // phi_AB, phi_BA on the identity map
+  p.warped = take(sizeof(float) * kBatch * vol);     // S(A, phi_AB), S(B, phi_BA)
+  if (ssd) {
+    p.tag = take(sizeof(float) * vol);
+    p.wtag = take(sizeof(float) * kBatch * vol);
+  } else {
+    p.zb = take(sizeof(float) * 5 * vol);
+  }
+  p.g = take(sizeof(double) * p.ng);
+  p.s = take(sizeof(double) * kBatch * 2 * p.ns);
+  p.m = take(sizeof(double) * p.nm);
+  p.count = take(sizeof(unsigned long long));
+  p.total = align256(off);
+  return p;
+}
+
+int check_loss_cfg(const oai_icon_loss_cfg* cfg) {
+  OAI_REQUIRE(cfg, "reg_icon_loss: null configuration");
+  OAI_REQUIRE(cfg->similarity == OAI_SIM_LNCC || cfg->similarity == OAI_SIM_SSD_ONLY_INTERPOLATED,
+              "reg_icon_loss: unknown similarity %d (0 = LNCC, 1 = ssd_only_interpolated)", cfg->similarity);
+  if (cfg->similarity == OAI_SIM_LNCC)
+    OAI_REQUIRE(cfg->sigma > 0 && lncc_radius(cfg->sigma) <= kLnccMaxRadius,
+                "reg_icon_loss: LNCC sigma %g outside (0, 12.5)", cfg->sigma);
+  OAI_REQUIRE(std::isfinite(cfg->delta) && cfg->delta > 0, "reg_icon_loss: delta %g must be positive", cfg->delta);
+  OAI_REQUIRE(std::isfinite(cfg->lmbda), "reg_icon_loss: lmbda must be finite");
+  return 0;
+}
+
+}  // namespace
+
+extern "C" size_t oai_reg_loss_workspace_bytes(oai_reg_t h, const oai_icon_loss_cfg* cfg) {
+  if (!h || check_loss_cfg(cfg)) return 0;
+  return loss_plan(h, *cfg).total;
+}
+
+extern "C" int oai_reg_icon_loss(oai_reg_t h, const oai_icon_loss_cfg* cfg, const float* noise, double* terms,
+                                 float* jac_det_BA, void* loss_ws, size_t loss_ws_bytes, const void* reg_ws,
+                                 size_t reg_ws_bytes, void* stream) {
+  RC(check_loss_cfg(cfg));
+  OAI_REQUIRE(h, "reg_icon_loss: null handle");
+  OAI_REQUIRE(noise && terms, "reg_icon_loss: null noise / terms");
+  OAI_REQUIRE(h->forwarded, "reg_icon_loss: no oai_reg_forward has run on this handle");
+  const LossPlan lp = loss_plan(h, *cfg);
+  OAI_REQUIRE(loss_ws && (reinterpret_cast<uintptr_t>(loss_ws) & 255) == 0 && loss_ws_bytes >= lp.total,
+              "reg_icon_loss: loss workspace of %zu bytes, 256-byte aligned, required (got %zu)", lp.total,
+              loss_ws_bytes);
+  RC(check_workspace(h, reg_ws, reg_ws_bytes, "reg_icon_loss"));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int* dims = h->dims;
+  const int D = dims[0], H = dims[1], W = dims[2];
+  const size_t vol = voxels(dims);
+  char* lw = static_cast<char*>(loss_ws);
+  char* arena = const_cast<char*>(static_cast<const char*>(reg_ws)) + h->scratch_bytes;
+  const float* pair = reinterpret_cast<const float*>(arena + h->pair_off);   // [A, B] at the network shape
+  float* phi = reinterpret_cast<float*>(lw + lp.phi);
+  float* warped = reinterpret_cast<float*>(lw + lp.warped);
+  double* g = reinterpret_cast<double*>(lw + lp.g);
+  double* s = reinterpret_cast<double*>(lw + lp.s);
+  double* m = reinterpret_cast<double*>(lw + lp.m);
+  auto* count = reinterpret_cast<unsigned long long*>(lw + lp.count);
+  const bool ssd = cfg->similarity == OAI_SIM_SSD_ONLY_INTERPOLATED;
+  nvtxRangePushA("oai.reg_icon_loss");
+  auto body = [&]() -> int {
+    Ctx c{h, st, false, arena, 0, nullptr, 0};
+    std::vector<Field> fields;
+    for (const FieldRef& r : h->fields) {
+      Field f;
+      f.p = reinterpret_cast<float*>(arena + r.off);
+      for (int a = 0; a < 3; ++a) f.dims[a] = r.dims[a];
+      fields.push_back(f);
+    }
+    if (ssd) RC(inbounds_tag_launch(reinterpret_cast<float*>(lw + lp.tag), D, H, W, st));
+    // phi_AB / phi_BA on the identity map and the warped images: direction k warps pair[k] onto pair[1 - k]
+    for (int k = 0; k < kBatch; ++k) {
+      RC(compose(c, fields, k, dims, pair + k * vol, dims, phi + k * 3 * vol, warped + k * vol));
+      if (ssd)
+        RC(compose(c, fields, k, dims, reinterpret_cast<const float*>(lw + lp.tag), dims, nullptr,
+                   reinterpret_cast<float*>(lw + lp.wtag) + k * vol));
+    }
+    for (int k = 0; k < kBatch; ++k) {
+      double* sk = s + static_cast<size_t>(k) * 2 * lp.ns;
+      if (ssd) {
+        RC(ssd_launch(warped + k * vol, reinterpret_cast<const float*>(lw + lp.wtag) + k * vol,
+                      pair + (1 - k) * vol, D, H, W, sk, sk + lp.ns, st));
+      } else {
+        LnccParams q{};
+        q.D = D; q.H = H; q.W = W;
+        q.I = warped + k * vol;
+        q.J = pair + (1 - k) * vol;
+        q.radius = lncc_radius(cfg->sigma);
+        double wsum = 0.0, w[2 * kLnccMaxRadius + 1];
+        for (int i = -q.radius; i <= q.radius; ++i) wsum += w[i + q.radius] = std::exp(-(i * i) / (2.0 * cfg->sigma * cfg->sigma));
+        for (int i = 0; i <= 2 * q.radius; ++i) q.taps[i] = static_cast<float>(w[i] / wsum);
+        q.zb = reinterpret_cast<float*>(lw + lp.zb);
+        q.partials = sk;
+        RC(lncc_launch(q, st));
+      }
+    }
+    GradIconParams gp{};
+    gp.D = D; gp.H = H; gp.W = W;
+    gp.noise = noise;
+    gp.delta = static_cast<float>(cfg->delta);
+    for (int dir = 0; dir < 2; ++dir) {   // phi_BA's fields (direction 1 of the batch) first, then phi_AB's
+      const int k = 1 - dir;
+      gp.nf[dir] = static_cast<int>(fields.size());
+      for (size_t f = 0; f < fields.size(); ++f) {
+        gp.u[dir][f] = fields[f].p + static_cast<size_t>(k) * 3 * voxels(fields[f].dims);
+        gp.ud[dir][f] = fields[f].dims[0]; gp.uh[dir][f] = fields[f].dims[1]; gp.uw[dir][f] = fields[f].dims[2];
+      }
+    }
+    gp.partials = g;
+    RC(gradicon_launch(gp, st));
+    JacobianParams jp{};
+    jp.D = D; jp.H = H; jp.W = W;
+    jp.phi_jac = phi + 3 * vol;   // losses.flips(phi_BA_vectorfield), as GradientICON.forward counts it
+    jp.phi_mag = phi;             // mean((identity_map - phi_AB_vectorfield) ** 2)
+    jp.det_out = jac_det_BA;
+    jp.count = count;
+    jp.mag_partials = m;
+    RC(jacobian_launch(jp, st));
+    LossFinishParams fp{};
+    fp.g = g; fp.ng = lp.ng;
+    fp.s = s; fp.ns = lp.ns; fp.ssd = ssd ? 1 : 0;
+    fp.m = m; fp.nm = lp.nm;
+    fp.count = count;
+    fp.nvox = static_cast<double>(vol);
+    fp.lmbda = cfg->lmbda;
+    fp.terms = terms;
+    return loss_finish_launch(fp, st);
+  };
+  const int rc = body();
+  nvtxRangePop();
+  return rc;
+}
+
+extern "C" int oai_jacobian_flips(const float* phi, const int* dims, float* det_out, long long* count_out,
+                                  void* stream) {
+  OAI_REQUIRE(phi && dims && count_out, "jacobian_flips: null pointer");
+  for (int a = 0; a < 3; ++a)
+    OAI_REQUIRE(dims[a] >= 2, "jacobian_flips: axis %d has %d samples (at least 2 needed)", a, dims[a]);
+  OAI_REQUIRE(static_cast<long long>((dims[2] + 31) / 32) * ((dims[1] + 7) / 8) * dims[0] < (1ll << 31),
+              "jacobian_flips: map too large");
+  JacobianParams jp{};
+  jp.D = dims[0]; jp.H = dims[1]; jp.W = dims[2];
+  jp.phi_jac = phi;
+  jp.det_out = det_out;
+  jp.count = reinterpret_cast<unsigned long long*>(count_out);
+  return jacobian_launch(jp, static_cast<cudaStream_t>(stream));
 }

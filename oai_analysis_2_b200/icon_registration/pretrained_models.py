@@ -2,7 +2,8 @@
 
 The reference builds GradientICON(TwoStep(TwoStep(Downsample(TwoStep(phi, psi)), xi), omega), similarity, lmbda) and
 at inference only uses the four tallUNet2 and the closures composing them; the loss terms GradientICON.forward also
-computes are discarded by register_pair, so they are not evaluated here."""
+computes are discarded by register_pair, so model(A, B) does not evaluate them.  GradICONModel.icon_loss computes them
+on request (similarity, inverse consistency, transform magnitude, folds) as a registration-quality check."""
 import os
 
 import numpy as np
@@ -10,6 +11,7 @@ import torch
 
 from .. import ops
 from ..segmentation.utils import load_checkpoint
+from .losses import LNCC, ICONLoss, similarity_config
 from .networks import TallUNet2
 
 # Module tree of OAI_knees_gradICON_model().regis_net as SURVEY App. B.2 recalls it:
@@ -19,6 +21,9 @@ from .networks import TallUNet2
 # make_network(..., include_last_step=True) layout TwoStep(TwoStep(Down(TwoStep(Down(phi), psi)), xi), omega).
 DEFAULT_PATHS = ("netPhi.netPhi.net.netPhi.net", "netPhi.netPhi.net.netPsi.net", "netPhi.netPsi.net", "netPsi.net")
 INPUT_SHAPE = [1, 1, 80, 192, 192]
+# GradientICON's similarity and lmbda of the knee model as recalled, not verified (SURVEY App. B.2, DESIGN.md §2)
+DEFAULT_SIMILARITY_SIGMA = 5
+DEFAULT_LMBDA = 1.5
 WEIGHTS_ENV = "OAI_B200_GRADICON_WEIGHTS"
 _UNET_PARAMS = ("downConvs.", "upConvs.", "batchNorms.", "lastConv.")
 
@@ -94,6 +99,9 @@ class GradICONModel:
         self._handle, self._handle_key = None, None
         self.phi_AB_vectorfield = None
         self.phi_BA_vectorfield = None
+        self.similarity = LNCC(sigma=DEFAULT_SIMILARITY_SIGMA)
+        self.lmbda = DEFAULT_LMBDA
+        self.delta = 1e-3
 
     # -- module-like surface
     def assign_identity_map(self, input_shape):
@@ -189,6 +197,21 @@ class GradICONModel:
         shape = tuple(image.shape[-3:])
         return self._stage().warp_image(image.reshape(shape).contiguous(), direction, out)
 
+    def icon_loss(self, image_A, image_B, noise=None):
+        """GradientICON.forward(A, B)'s ICONLoss for the pair at the network shape ([1,1,D,H,W] or [D,H,W] float32
+        cuda, as forward takes them): registers it (phi_AB / phi_BA are updated as by model(A, B)) and returns
+        ICONLoss(all_loss, inverse_consistency_loss, similarity_loss, transform_magnitude, flips) of 0-d float64 CUDA
+        tensors, with self.similarity and self.lmbda.  noise: N(0, 1) of the identity map's shape [1,3,D,H,W]; when
+        None it is drawn as icon draws it (torch.randn on the CPU default generator), so torch.manual_seed reproduces
+        icon's Iepsilon."""
+        self.forward(image_A, image_B)
+        if noise is None:
+            noise = torch.randn(*self.identity_map.shape)
+        noise = noise.to(device=self.device, dtype=torch.float32).reshape(3, *self.input_shape[2:]).contiguous()
+        kind, sigma = similarity_config(self.similarity)
+        terms, _ = self._stage().icon_loss(noise, kind, sigma, self.lmbda, self.delta)
+        return ICONLoss(*terms.unbind())
+
     def _eval_on_identity(self, field, coords):
         if field is None:
             raise RuntimeError("call the model on an image pair first")
@@ -203,11 +226,18 @@ class GradICONModel:
         return self._eval_on_identity(self.phi_BA_vectorfield, coords)
 
 
-def OAI_knees_gradICON_model(pretrained=True, weights_path=None):
+def OAI_knees_gradICON_model(pretrained=True, weights_path=None, similarity=None, lmbda=None):
     """pretrained_models.OAI_knees_gradICON_model.  The reference downloads the checkpoint from a GitHub release;
-    here `weights_path` (or $OAI_B200_GRADICON_WEIGHTS) must point at that file when pretrained=True."""
+    here `weights_path` (or $OAI_B200_GRADICON_WEIGHTS) must point at that file when pretrained=True.
+    similarity (losses.LNCC(sigma) or losses.ssd_only_interpolated) and lmbda override the loss configuration that
+    icon_loss uses; registration itself does not depend on them."""
     net = GradICONModel()
     net.assign_identity_map(INPUT_SHAPE)
+    if similarity is not None:
+        similarity_config(similarity)   # raises for anything the library cannot compute
+        net.similarity = similarity
+    if lmbda is not None:
+        net.lmbda = float(lmbda)
     if pretrained:
         path = weights_path or os.environ.get(WEIGHTS_ENV)
         if not path or not os.path.isfile(path):

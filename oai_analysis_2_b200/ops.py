@@ -274,6 +274,9 @@ def reg_parse_tree(state_dict):
     return buf.value.decode()
 
 
+SIM_LNCC, SIM_SSD_ONLY_INTERPOLATED = 0, 1   # oai_icon_loss_cfg.similarity
+
+
 class RegHandle:
     """oai_reg_create / oai_reg_forward / oai_reg_destroy: register_pair on the GradICON cascade behind one handle.
     The workspace (concatenation buffers, intermediate images, the cascade's displacement fields) is owned here and
@@ -331,6 +334,56 @@ class RegHandle:
         check(lib.oai_reg_warp_image(self._h, ptr(image), ptr(_dims(*shape)), int(direction), ptr(out), ptr(self._ws),
                                      c_size(self._ws.numel()), stream_ptr()), "reg_warp_image")
         return out
+
+    def loss_workspace_bytes(self, similarity=SIM_LNCC, sigma=5.0, lmbda=1.5, delta=1e-3):
+        cfg = icon_loss_cfg(similarity, sigma, lmbda, delta)
+        n = int(lib.oai_reg_loss_workspace_bytes(self._h, ctypes.byref(cfg)))
+        if n == 0:   # a refused configuration: the call reports why before touching anything
+            check(lib.oai_reg_icon_loss(self._h, ctypes.byref(cfg), None, None, None, None, c_size(0), None,
+                                        c_size(0), None), "reg_icon_loss")
+        return n
+
+    def icon_loss(self, noise, similarity=SIM_LNCC, sigma=5.0, lmbda=1.5, delta=1e-3, want_det=False, terms=None,
+                  det=None):
+        """GradientICON.forward's loss terms for the last forward (oai_reg_icon_loss).  noise: float32 cuda
+        [3, *net_dims] (or [1, 3, *net_dims]) of N(0, 1) values.  Returns (terms, det): terms float64 [5] in ICONLoss
+        order (all, inverse consistency, similarity, transform magnitude, flips), det the dV map of phi_BA
+        [D-1, H-1, W-1] when want_det (else None).  The loss workspace is owned by the handle and only grows, so a
+        CUDA graph captured over this call keeps valid pointers."""
+        d = self.net_dims
+        assert noise.dtype == torch.float32 and noise.is_cuda and noise.is_contiguous() and noise.numel() == 3 * math.prod(d)
+        need = self.loss_workspace_bytes(similarity, sigma, lmbda, delta)
+        if getattr(self, "_loss_ws", None) is None or self._loss_ws.numel() < need:
+            self._loss_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        if terms is None:
+            terms = torch.empty(5, dtype=torch.float64, device=self.device)
+        if want_det and det is None:
+            det = torch.empty(tuple(v - 1 for v in d), dtype=torch.float32, device=self.device)
+        cfg = icon_loss_cfg(similarity, sigma, lmbda, delta)
+        check(lib.oai_reg_icon_loss(self._h, ctypes.byref(cfg), ptr(noise), ptr(terms), ptr(det if want_det else None),
+                                    ptr(self._loss_ws), c_size(self._loss_ws.numel()), ptr(self._ws),
+                                    c_size(self._ws.numel()), stream_ptr()), "reg_icon_loss")
+        return terms, (det if want_det else None)
+
+
+class _IconLossCfg(ctypes.Structure):
+    _fields_ = [("similarity", c_int), ("sigma", c_double), ("lmbda", c_double), ("delta", c_double)]
+
+
+def icon_loss_cfg(similarity=SIM_LNCC, sigma=5.0, lmbda=1.5, delta=1e-3):
+    """oai_icon_loss_cfg: similarity SIM_LNCC (with sigma) or SIM_SSD_ONLY_INTERPOLATED, lmbda, delta."""
+    return _IconLossCfg(int(similarity), float(sigma), float(lmbda), float(delta))
+
+
+def jacobian_flips(phi, det=False):
+    """losses.flips' fold count of one map phi [3, D, H, W] (or [1, 3, D, H, W]) float32 cuda: returns the number of
+    cells with dV < 0 as a 0-d int64 cuda tensor, and with det=True also the dV map [D-1, H-1, W-1]."""
+    assert phi.dtype == torch.float32 and phi.is_cuda and phi.is_contiguous() and phi.shape[-4] == 3
+    shape = tuple(int(v) for v in phi.shape[-3:])
+    count = torch.empty((), dtype=torch.int64, device=phi.device)
+    dv = torch.empty(tuple(max(v - 1, 0) for v in shape), dtype=torch.float32, device=phi.device) if det else None
+    check(lib.oai_jacobian_flips(ptr(phi), ptr(_dims(*shape)), ptr(dv), ptr(count), stream_ptr()), "jacobian_flips")
+    return (count, dv) if det else count
 
 
 # ------------------------------------------------------------------------------------------------ registration
