@@ -381,6 +381,31 @@ OAI_API int oai_reg_icon_loss(oai_reg_t handle, const oai_icon_loss_cfg* cfg, co
  * device float32 [D-1][H-1][W-1].  Every axis needs at least 2 samples. */
 OAI_API int oai_jacobian_flips(const float* phi, const int* dims, float* det_out, long long* count_out, void* stream);
 
+/* Segmentation quality: overlap and surface distances of two masks A and B on one grid dims = {D, H, W} (z, y, x),
+ * every axis 1 to 512 voxels; spacing_xyz = {sx, sy, sz} in mm, positive and finite.  The definitions are medpy's
+ * dc / assd / hd / hd95:
+ *   surface  dM = M & ~binary_erosion(M, 6-connected cross, border_value=0): mask voxels on a volume face are surface;
+ *   d_AB     = EDT to dB at the voxels of dA, d_BA likewise, in mm between voxel centres;
+ *   dice     = 2|A & B| / (|A| + |B|);  assd = (mean d_AB + mean d_BA) / 2;  hd = max(max d_AB, max d_BA);
+ *   hd95     = np.percentile(np.hstack((d_AB, d_BA)), 95), numpy's linear interpolation (an exact order statistic).
+ * dice is NaN when both masks are empty; assd, hd, hd95 and the means and maxima are NaN when either is empty.
+ * workspace: 256-byte aligned device memory of oai_seg_quality_workspace_bytes(dims) bytes (0 for unsupported dims);
+ * it serves both calls.  Fixed-order reductions (equal inputs give bitwise equal terms); no host synchronisation, no
+ * allocation. */
+OAI_API size_t oai_seg_quality_workspace_bytes(const int* dims);
+/* scipy.ndimage.distance_transform_edt(~feature, sampling=(sz, sy, sx)): out[v] = distance in mm from voxel v to the
+ * nearest voxel with feature[v] != 0 (+inf everywhere when there is none).  feature: device uint8 [dims]; out: device
+ * float32 [dims]. */
+OAI_API int oai_distance_transform(const uint8_t* feature, const int* dims, const double* spacing_xyz, float* out,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+/* mask_a, mask_b: device uint8 [dims], non-zero = inside.
+ * terms: device double[8] = {dice, assd, hd95, hd, mean d_AB, mean d_BA, max d_AB, max d_BA};
+ * counts: device int64[5] = {|A|, |B|, |A & B|, |dA|, |dB|};
+ * dist_to_B / dist_to_A (optional, NULL to skip): device float32 [dims], the EDT maps to dB and to dA in mm. */
+OAI_API int oai_surface_metrics(const uint8_t* mask_a, const uint8_t* mask_b, const int* dims,
+                                const double* spacing_xyz, double* terms, long long* counts, float* dist_to_B,
+                                float* dist_to_A, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------------
  * ITK-semantics warps  (reference: oai_analysis/dask_processing.py:95-111 deform_probmap_delayed,
  * test/test_all.py:42-52; transform = R_A o DisplacementFieldTransform o R_B^-1 built by create_itk_transform)

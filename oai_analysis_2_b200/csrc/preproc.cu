@@ -7,37 +7,15 @@
 // is read four times and written once (20 B / voxel).
 #include "../../include/oai_b200.h"
 #include "api_common.h"
+#include "radix_select.cuh"
 
 namespace oai {
 namespace {
 
-constexpr int kTargets = 4;  // floor / ceil order statistics of the two percentiles
-struct SelectState {
-  unsigned long long rank[kTargets];   // remaining rank inside the surviving prefix
-  unsigned int prefix[kTargets];       // selected high bits so far
-  unsigned int hist1[2048];
-  unsigned int hist2[kTargets][2048];
-  unsigned int hist3[kTargets][1024];
-  float frac[2];                       // interpolation weights (numpy's gamma) of the two percentiles
-  double window[2];                    // result: window_min, window_max
-};
-
-__device__ __forceinline__ unsigned int float_key(float v) {
-  const unsigned int u = __float_as_uint(v);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);  // monotone: key order == float order
-}
-__device__ __forceinline__ float key_float(unsigned int k) {
-  return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
-}
-
 __global__ void __launch_bounds__(256) window_init_kernel(SelectState* s, long long n, double p_lo, double p_hi) {
   const int t = threadIdx.x;
-  for (int i = t; i < 2048; i += 256) {
-    s->hist1[i] = 0;
-    for (int k = 0; k < kTargets; ++k) s->hist2[k][i] = 0;
-    if (i < 1024)
-      for (int k = 0; k < kTargets; ++k) s->hist3[k][i] = 0;
-  }
+  select_reset(s);
+  if (t == 0) s->n = n;
   if (t < 2) {
     // numpy >= 2 on a float32 array (NEP 50: the Python-float percentile and the integer count are "weak" and take the
     // array's dtype): q = float32(p) / float32(100); virtual index = float32(n - 1) * q; previous = floor, next =
@@ -59,102 +37,25 @@ __global__ void __launch_bounds__(256) window_init_kernel(SelectState* s, long l
     s->rank[2 * t] = k0;
     s->rank[2 * t + 1] = k1;
     s->frac[t] = gamma;
-    s->prefix[2 * t] = s->prefix[2 * t + 1] = 0;
   }
 }
 
-// PASS 0: top 11 bits of every key; PASS 1 / 2: next 11 / last 10 bits of the keys whose higher bits match a target
-template <int PASS>
-__global__ void __launch_bounds__(512) window_hist_kernel(const float* __restrict__ in, long long n, SelectState* s) {
-  constexpr int BINS = PASS == 2 ? 1024 : 2048;
-  constexpr int NH = PASS == 0 ? 1 : kTargets;
-  __shared__ unsigned int sh[NH][BINS];
-  for (int i = threadIdx.x; i < NH * BINS; i += blockDim.x) (&sh[0][0])[i] = 0;
-  unsigned int pre[kTargets] = {0, 0, 0, 0};
-  if (PASS > 0) {
-#pragma unroll
-    for (int k = 0; k < kTargets; ++k) pre[k] = s->prefix[k];
-  }
-  __syncthreads();
-  const long long n4 = n / 4;
-  auto visit = [&](float v) {
-    const unsigned int key = float_key(v);
-    if (PASS == 0) {
-      // smooth volumes put most keys of a warp into a handful of bins: one atomic per distinct bin of the warp
-      const unsigned int bin = key >> 21, act = __activemask();
-      const unsigned int same = __match_any_sync(act, bin);
-      if ((__ffs(same) - 1) == static_cast<int>(threadIdx.x & 31)) atomicAdd(&sh[0][bin], __popc(same));
-    } else {
-      const unsigned int hi = PASS == 1 ? key >> 21 : key >> 10;
-      const unsigned int bin = PASS == 1 ? (key >> 10) & 2047u : key & 1023u;
-#pragma unroll
-      for (int k = 0; k < kTargets; ++k)
-        if (hi == pre[k]) atomicAdd(&sh[PASS == 0 ? 0 : k][bin], 1u);
-    }
-  };
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n4;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const float4 v = __ldg(reinterpret_cast<const float4*>(in) + i);
-    visit(v.x); visit(v.y); visit(v.z); visit(v.w);
-  }
-  if (blockIdx.x == 0)
-    for (long long i = 4 * n4 + threadIdx.x; i < n; i += blockDim.x) visit(__ldg(in + i));
-  __syncthreads();
-  unsigned int* g = PASS == 0 ? s->hist1 : (PASS == 1 ? &s->hist2[0][0] : &s->hist3[0][0]);
-  for (int i = threadIdx.x; i < NH * BINS; i += blockDim.x) {
-    const unsigned int c = (&sh[0][0])[i];
-    if (c) atomicAdd(g + i, c);
-  }
-}
-
-// one warp per target: find the bin holding the remaining rank, extend the prefix
-template <int PASS>
-__global__ void __launch_bounds__(32 * kTargets) window_pick_kernel(SelectState* s, float out_min, float out_max) {
-  constexpr int BINS = PASS == 2 ? 1024 : 2048;
-  constexpr int BITS = PASS == 2 ? 10 : 11;
-  const int k = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const unsigned int* h = PASS == 0 ? s->hist1 : (PASS == 1 ? s->hist2[k] : s->hist3[k]);
-  unsigned long long rank = s->rank[k], base = 0;
-  int found = -1;
-  for (int b0 = 0; b0 < BINS && found < 0; b0 += 32) {
-    const unsigned int c = h[b0 + lane];
-    unsigned long long incl = c;  // inclusive scan over the warp
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const unsigned long long o = __shfl_up_sync(0xffffffffu, incl, d);
-      if (lane >= d) incl += o;
-    }
-    const bool here = base + incl > rank;
-    const unsigned int m = __ballot_sync(0xffffffffu, here);
-    if (m) {
-      const int l = __ffs(m) - 1;
-      const unsigned long long before = base + __shfl_sync(0xffffffffu, incl, l) - __shfl_sync(0xffffffffu, (unsigned long long)c, l);
-      found = b0 + l;
-      rank -= before;
-    } else {
-      base += __shfl_sync(0xffffffffu, incl, 31);
-    }
-  }
-  if (found < 0) found = BINS - 1;  // unreachable for rank < n
-  if (lane == 0) {
-    s->rank[k] = rank;
-    s->prefix[k] = (s->prefix[k] << BITS) | static_cast<unsigned int>(found);
-  }
-  if (PASS == 2) {
-    __syncthreads();
-    if (threadIdx.x < 2) {  // numpy _lerp in float32: a + (b - a) * t, taken from the other end for t >= 0.5
-      const float a = key_float(s->prefix[2 * threadIdx.x]), b = key_float(s->prefix[2 * threadIdx.x + 1]);
-      const float t = s->frac[threadIdx.x], d = __fsub_rn(b, a);
-      const float r = t >= 0.5f ? __fsub_rn(b, __fmul_rn(d, __fsub_rn(1.f, t))) : __fadd_rn(a, __fmul_rn(d, t));
-      s->window[threadIdx.x] = static_cast<double>(r);
-    }
-  }
+// numpy _lerp in float32 of percentile i from the selected order statistics: a + (b - a) * t, taken from the other end
+// for t >= 0.5
+__device__ __forceinline__ float window_bound(const SelectState* s, int i) {
+  const float a = key_float(s->prefix[2 * i]), b = key_float(s->prefix[2 * i + 1]);
+  const float t = s->frac[i], d = __fsub_rn(b, a);
+  return t >= 0.5f ? __fsub_rn(b, __fmul_rn(d, __fsub_rn(1.f, t))) : __fadd_rn(a, __fmul_rn(d, t));
 }
 
 __global__ void __launch_bounds__(256) window_apply_kernel(const float* __restrict__ in, long long n,
-                                                           const SelectState* __restrict__ s, float out_min,
+                                                           SelectState* __restrict__ s, float out_min,
                                                            float out_max, float* __restrict__ out) {
-  const float wmin = static_cast<float>(s->window[0]), wmax = static_cast<float>(s->window[1]);
+  const float wmin = window_bound(s, 0), wmax = window_bound(s, 1);
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    s->window[0] = static_cast<double>(wmin);
+    s->window[1] = static_cast<double>(wmax);
+  }
   // itk::Functor::IntensityWindowingTransform: factor / offset in RealType (double)
   const double factor = (static_cast<double>(out_max) - static_cast<double>(out_min)) /
                         (static_cast<double>(wmax) - static_cast<double>(wmin));
@@ -203,18 +104,7 @@ extern "C" int oai_intensity_window(const float* in, long long n, double perc_lo
   const unsigned grid = static_cast<unsigned>(num_sms()) * 4;
   window_init_kernel<<<1, 256, 0, st>>>(s, n, perc_lo, perc_hi);
   if (int rc = launched("window_init_kernel")) return rc;
-  window_hist_kernel<0><<<grid, 512, 0, st>>>(in, n, s);
-  if (int rc = launched("window_hist_kernel<0>")) return rc;
-  window_pick_kernel<0><<<1, 32 * kTargets, 0, st>>>(s, out_min, out_max);
-  if (int rc = launched("window_pick_kernel<0>")) return rc;
-  window_hist_kernel<1><<<grid, 512, 0, st>>>(in, n, s);
-  if (int rc = launched("window_hist_kernel<1>")) return rc;
-  window_pick_kernel<1><<<1, 32 * kTargets, 0, st>>>(s, out_min, out_max);
-  if (int rc = launched("window_pick_kernel<1>")) return rc;
-  window_hist_kernel<2><<<grid, 512, 0, st>>>(in, n, s);
-  if (int rc = launched("window_hist_kernel<2>")) return rc;
-  window_pick_kernel<2><<<1, 32 * kTargets, 0, st>>>(s, out_min, out_max);
-  if (int rc = launched("window_pick_kernel<2>")) return rc;
+  if (int rc = select_launch(in, s, grid, st)) return rc;
   window_apply_kernel<<<grid * 2, 256, 0, st>>>(in, n, s, out_min, out_max, out);
   return launched("window_apply_kernel");
 }

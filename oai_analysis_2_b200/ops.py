@@ -386,6 +386,48 @@ def jacobian_flips(phi, det=False):
     return (count, dv) if det else count
 
 
+# ------------------------------------------------------------------------------------------------ segmentation quality
+def _mask_u8(m):
+    assert m.is_cuda and m.dim() == 3 and m.dtype in (torch.bool, torch.uint8), "expected a bool/uint8 cuda [D,H,W]"
+    return (m.view(torch.uint8) if m.dtype == torch.bool else m).contiguous()
+
+
+def _seg_quality_ws(device, shape):
+    dims = _dims(*shape)
+    nbytes = int(lib.oai_seg_quality_workspace_bytes(ptr(dims)))
+    return dims, _scratch_buf(device, "seg_quality", nbytes), nbytes
+
+
+def distance_transform(feature, spacing_xyz):
+    """scipy.ndimage.distance_transform_edt(~feature, sampling=(sz, sy, sx)) on the device, exact: feature bool/uint8
+    cuda [D,H,W] -> float32 [D,H,W], the distance in mm to the nearest non-zero voxel (+inf when there is none)."""
+    f = _mask_u8(feature)
+    out = torch.empty(f.shape, dtype=torch.float32, device=f.device)
+    dims, ws, nbytes = _seg_quality_ws(f.device, f.shape)
+    sp = np.asarray(spacing_xyz, dtype=np.float64)
+    check(lib.oai_distance_transform(ptr(f), ptr(dims), ptr(sp), ptr(out), ptr(ws), c_size(nbytes), stream_ptr()),
+          "distance_transform")
+    return out
+
+
+def surface_metrics(mask_a, mask_b, spacing_xyz, maps=False):
+    """Overlap and surface distances of two bool/uint8 cuda masks [D,H,W] (medpy's dc / assd / hd95 / hd): returns
+    (terms float64[8] = dice, assd, hd95, hd, mean d_AB, mean d_BA, max d_AB, max d_BA;  counts int64[5] = |A|, |B|,
+    |A&B|, |dA|, |dB|), and with maps=True also the EDT maps (dist_to_B, dist_to_A) float32 [D,H,W] in mm.  Everything
+    stays on the device; nothing synchronises."""
+    a, b = _mask_u8(mask_a), _mask_u8(mask_b)
+    assert a.shape == b.shape and a.device == b.device, "masks must share one grid"
+    terms = torch.empty(8, dtype=torch.float64, device=a.device)
+    counts = torch.empty(5, dtype=torch.int64, device=a.device)
+    to_b = torch.empty(a.shape, dtype=torch.float32, device=a.device) if maps else None
+    to_a = torch.empty(a.shape, dtype=torch.float32, device=a.device) if maps else None
+    dims, ws, nbytes = _seg_quality_ws(a.device, a.shape)
+    sp = np.asarray(spacing_xyz, dtype=np.float64)
+    check(lib.oai_surface_metrics(ptr(a), ptr(b), ptr(dims), ptr(sp), ptr(terms), ptr(counts), ptr(to_b), ptr(to_a),
+                                  ptr(ws), c_size(nbytes), stream_ptr()), "surface_metrics")
+    return (terms, counts, to_b, to_a) if maps else (terms, counts)
+
+
 # ------------------------------------------------------------------------------------------------ registration
 def _dims(*v):
     return np.asarray(v, dtype=np.int32)
