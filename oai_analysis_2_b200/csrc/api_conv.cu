@@ -73,7 +73,8 @@ int build_chunks(const ConvSpec& s, Plan* pl) {
   return 0;
 }
 
-int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0) {
+// tw: M tile width of a kh-shared layer (8, 16 or 32); the packed weights do not depend on it
+int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0, int tw = 32) {
   const int D = s.D, H = s.H, W = s.W, c0 = s.c0, c1 = s.c1, cout = s.cout, pointwise = s.kind, flags = s.flags;
   OAI_REQUIRE(D > 0 && H > 0 && W > 0 && c0 > 0 && c1 >= 0 && cout > 0, "conv plan: bad dims");
   OAI_REQUIRE(c0 % 8 == 0 && c1 % 8 == 0, "conv plan: channel counts must be multiples of 8 (got %d,%d)", c0, c1);
@@ -86,9 +87,11 @@ int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0) {
   OAI_REQUIRE((!s.split0 || c0 % 32 == 0) && (!s.split1 || c1 % 64 == 0) && (c1 == 0 || c0 % 64 == 0),
               "conv plan: split / concatenated sources need 64-channel multiples (got %d,%d)", c0, c1);
   pl->TW = W < 128 ? W : 128;
-  OAI_REQUIRE(128 % pl->TW == 0 && W % pl->TW == 0, "conv plan: W=%d must divide or be a multiple of 128", W);
   pl->TH = 128 / pl->TW;
-  OAI_REQUIRE(H % pl->TH == 0, "conv plan: H=%d not a multiple of the %d-row M tile", H, pl->TH);
+  if (!(flags & kConvFlagKhShared)) {
+    OAI_REQUIRE(128 % pl->TW == 0 && W % pl->TW == 0, "conv plan: W=%d must divide or be a multiple of 128", W);
+    OAI_REQUIRE(H % pl->TH == 0, "conv plan: H=%d not a multiple of the %d-row M tile", H, pl->TH);
+  }
   // 3x3x3 layers split cout into 128-wide N tiles: each tile then stacks the three kd taps of an input slice (N = 256 +
   // 128) and keeps R = 4 accumulators, which halves the weight bytes streamed per output compared with a 256-wide
   // tile limited to R = 2 by the 512 TMEM columns.  Pointwise layers keep 256-wide tiles.
@@ -136,6 +139,17 @@ int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0) {
     pl->wblock_bytes = pl->cph * rb;
     pl->nblk = nch;
     pl->n_wbuf = 3;
+  } else if (flags & kConvFlagKhShared) {
+    OAI_REQUIRE(pl->cph <= 64 && rb == 128 && (tw == 8 || tw == 16 || tw == 32) && W >= tw && H >= 128 / tw,
+                "conv plan: kh-shared mode needs cout <= 64, 64-channel chunks and a grid of at least one %d-wide tile "
+                "(cout=%d, %dx%d)", tw, cout, H, W);
+    pl->mode = kModeKhShared;
+    pl->kd_per_block = 3;
+    pl->wblock_bytes = 9 * pl->cph * rb;
+    pl->nblk = nch * 3;
+    pl->n_wbuf = 2;
+    pl->TW = tw;
+    pl->TH = 128 / tw;
   } else if (pl->TW == 128 && pl->cph <= 64 && !(flags & kFlagForcePerTap)) {
     pl->mode = kModeRowShared;
     pl->kd_per_block = 3;
@@ -158,7 +172,7 @@ int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0) {
     pl->nkh = 3;
     pl->n_wbuf = 1;
   }
-  pl->astage_bytes = (pl->mode == kModeRowShared ? 130 : 128) * rb * pl->nkh;
+  pl->astage_bytes = (pl->mode == kModeRowShared ? 130 : pl->mode == kModeKhShared ? 128 + 2 * pl->TW : 128) * rb * pl->nkh;
   pl->astage_stride = (pl->astage_bytes + 1023u) & ~1023u;
   const size_t wstride = (static_cast<size_t>(pl->wblock_bytes) * pl->nkh + 1023u) & ~size_t(1023);
   // Stationary weights: a k2s2 unit is one K pass over a 128-voxel tile, so streaming its weight blocks per unit costs
@@ -319,8 +333,11 @@ int conv_pack_weights(const ConvSpec& s, const float* w, void* dst, size_t dst_b
         uint8_t* blk = out + ((static_cast<size_t>(nh) * ngroups + tg) * pl.nblk + b) * pl.wblock_bytes;
         // decode the block exactly as the kernel does: chunk c, and the taps whose rows are stacked in it
         int c, kh = 0, kw0 = 0, nkw = 1, kdlo = 0, nkd = 1;
+        const bool kh_inner = pl.mode == kModeKhShared;   // the three sub-blocks step kh instead of kw
         if (pl.mode == kModeRowShared) {
           c = b / 3; kh = b % 3; nkw = 3; nkd = 3;
+        } else if (kh_inner) {
+          c = b / 3; kw0 = b % 3; nkw = 3; nkd = 3;
         } else if (pl.mode == kModePerTap && pl.kd_per_block == 3) {
           c = b / 9; const int r = b % 9; kh = r / 3; kw0 = r % 3; nkd = 3;
         } else if (pl.mode == kModePerTap) {
@@ -337,6 +354,7 @@ int conv_pack_weights(const ConvSpec& s, const float* w, void* dst, size_t dst_b
             int tap;
             if (pl.mode == kModeUp2) tap = tg * pl.R + ti;
             else if (s.kind == 1) tap = 0;
+            else if (kh_inner) tap = ((kdlo + nkd - 1 - ti) * 3 + kh + kwi) * 3 + kw0;
             else tap = ((kdlo + nkd - 1 - ti) * 3 + kh) * 3 + kw0 + kwi;
             for (int co = 0; co < pl.cph; ++co) {
               const int r = (kwi * nstack + ti) * pl.cph + co;
@@ -356,18 +374,38 @@ int conv_pack_weights(const ConvSpec& s, const float* w, void* dst, size_t dst_b
 
 int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
   const int D = s.D, H = s.H, W = s.W, c0 = s.c0, c1 = s.c1, cout = s.cout;
-  // region = {d_lo, d_cnt, h_lo, h_cnt}: the output sub-box to compute (full rows in w); h range is widened to whole
-  // M-tile rows.  Everything outside is dead halo the caller never reads.
-  int d_lo = 0, d_cnt = D, h_lo = 0, h_cnt = H;
+  // region = {d_lo, d_cnt, h_lo, h_cnt} (+ a.w_lo, a.w_cnt): the output sub-box to compute.  Everything outside is dead
+  // halo the caller never reads.  Without a w range, rows are computed whole and the h range is widened to whole
+  // M-tile rows; a kh-shared layer places its tiles from (h_lo, w_lo) instead.
+  const bool kh_shared = (s.flags & kConvFlagKhShared) != 0;
+  int d_lo = 0, d_cnt = D, h_lo = 0, h_cnt = H, w_lo = 0, w_cnt = W;
   if (a.region) {
     d_lo = a.region[0]; d_cnt = a.region[1]; h_lo = a.region[2]; h_cnt = a.region[3];
     OAI_REQUIRE(d_lo >= 0 && d_cnt >= 1 && d_lo + d_cnt <= D && h_lo >= 0 && h_cnt >= 1 && h_lo + h_cnt <= H,
                 "conv: region [%d,+%d)x[%d,+%d) outside %dx%d", d_lo, d_cnt, h_lo, h_cnt, D, H);
   }
+  if (a.w_cnt) {
+    w_lo = a.w_lo; w_cnt = a.w_cnt;
+    OAI_REQUIRE(kh_shared, "conv: a w range needs a layer packed for kh-shared mode");
+    OAI_REQUIRE(w_lo >= 0 && w_cnt >= 1 && w_lo + w_cnt <= W, "conv: w range [%d,+%d) outside W=%d", w_lo, w_cnt, W);
+  }
+  // kh-shared tile width: the fewest M tiles over the box, the widest on a tie (dc1's 96 x 96 box: 72 tiles at every
+  // width; 32 x 4 and 8 x 16 tiles measured the same, 7.98 / 7.90 ms, though the 8-wide box is 25 % fewer bytes)
+  int tw = 32, ntile = 0;
+  if (kh_shared)
+    for (int t = 32; t >= 8; t /= 2) {
+      if (t > W || 128 / t > H) continue;
+      const int n = ((w_cnt + t - 1) / t) * ((h_cnt + 128 / t - 1) / (128 / t));
+      if (ntile == 0 || n < ntile) { ntile = n; tw = t; }
+    }
   Plan pl;
-  if (make_plan(s, &pl, d_cnt)) return 1;
-  const int hp_lo = h_lo / pl.TH;
-  const int hp_cnt = (h_lo + h_cnt + pl.TH - 1) / pl.TH - hp_lo;
+  if (make_plan(s, &pl, d_cnt, tw)) return 1;
+  int tile_h_lo = h_lo, nph = (h_cnt + pl.TH - 1) / pl.TH, npw = (w_cnt + pl.TW - 1) / pl.TW;
+  if (!kh_shared) {   // whole M-tile rows of whole-row (or whole-grid-aligned) tiles
+    tile_h_lo = h_lo / pl.TH * pl.TH;
+    nph = (h_lo + h_cnt + pl.TH - 1) / pl.TH - h_lo / pl.TH;
+    npw = W / pl.TW;
+  }
   const HeadFuse* head = a.head;
   OAI_REQUIRE(a.src0 && a.wpack && a.bias, "conv: null pointer");
   OAI_REQUIRE(!head || (pl.cph == 64 && pl.nhalf == 1), "conv head: the fused head needs a 64-channel layer");
@@ -403,9 +441,9 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
   p.out = a.out;
   p.obase = a.obase; p.osN = a.osN; p.osD = a.osD; p.osH = a.osH; p.osW = a.osW;
   p.out_split = a.out_split; p.out_lo_off = a.out_lo_off;
-  p.d_lo = d_lo; p.d_cnt = d_cnt; p.hp_lo = hp_lo; p.hp_cnt = hp_cnt;
+  p.d_lo = d_lo; p.d_cnt = d_cnt; p.h_lo = tile_h_lo; p.nph = nph; p.w_lo = kh_shared ? w_lo : 0; p.npw = npw;
   p.Rd = pl.Rd; p.up_groups = pl.up_groups;
-  p.nunits = a.NT * ((d_cnt + pl.Rd - 1) / pl.Rd) * (hp_cnt * (W / pl.TW)) * pl.up_groups * pl.nhalf;
+  p.nunits = a.NT * ((d_cnt + pl.Rd - 1) / pl.Rd) * (nph * npw) * pl.up_groups * pl.nhalf;
   if (pl.mode == kModeUp2) {
     // tap (a,b,c) lands on voxel (2z+a, 2y+b, 2x+c): osW is the element pitch of TWO output voxels (set by the caller)
     const long long vox = a.osW / 2;
@@ -416,7 +454,7 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
 
   OAI_REQUIRE(pl.mode != kModeUp2 || (c1 == 0 && !head), "conv: up2 mode takes one source and no fused head");
   const int bw = pl.mode == kModeRowShared ? 130 : pl.TW;
-  const int bh = pl.TH * pl.nkh;
+  const int bh = pl.mode == kModeKhShared ? pl.TH + 2 : pl.TH * pl.nkh;
   CUtensorMap tm0, tm1;
   if (make_act_tmap(&tm0, a.src0, s.split0 ? 2 * c0 : c0, W, H, D, a.NT, bw, bh, s.fmt, pl.row_bytes)) return 1;
   if (a.src1) {
@@ -434,9 +472,9 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
     }
     pe = &g_prof[g_prof_used++];
     const double taps = s.kind == 0 ? 27.0 : (s.kind == 1 ? 1.0 : 8.0);
-    pe->flops = 2.0 * a.NT * D * H * W * static_cast<double>(cout) * (c0 + c1) * taps;
-    // issued to the tensor pipe: computed rows x every K chunk listed (split-precision terms included)
-    pe->exec_flops = 2.0 * a.NT * static_cast<double>(d_cnt) * hp_cnt * pl.TH * W * static_cast<double>(cout) * taps *
+    pe->flops = 2.0 * a.NT * D * H * W * static_cast<double>(cout) * (c0 + c1) * taps * a.flop_share;
+    // issued to the tensor pipe: computed M tiles x every K chunk listed (split-precision terms included)
+    pe->exec_flops = 2.0 * a.NT * static_cast<double>(d_cnt) * nph * npw * 128 * static_cast<double>(cout) * taps *
                      (static_cast<double>(pl.nch) * pl.k16 * 16);
     prof_record(pe->a, st);
   }

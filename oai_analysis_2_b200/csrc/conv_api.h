@@ -8,6 +8,10 @@
 
 namespace oai {
 
+// ConvSpec::flags bit: pack and run a 3x3x3 layer in kh-shared mode (conv_igemm.cuh), whose M tiles may cover any
+// (h, w) box; the weight blocks are ordered (chunk, kw) with the 3 kh x 3 kd taps inside.
+constexpr int kConvFlagKhShared = 256;
+
 struct ConvSpec {
   int D, H, W;         // layer grid (the INPUT grid for kind 2)
   int c0, c1;          // logical channels of source 0 / source 1 (skip connection; 0 if absent)
@@ -33,6 +37,8 @@ struct ConvLaunch {
   int out_split;                        // also write the lo plane out_lo_off elements after the hi plane
   long long out_lo_off;
   const int* region;                    // {d_lo, d_cnt, h_lo, h_cnt} or nullptr
+  int w_lo = 0, w_cnt = 0;              // w range of the region (kConvFlagKhShared layers only; 0: full rows)
+  double flop_share = 1.0;              // part of the layer's algorithmic MACs the profile books on this launch
   const HeadFuse* head;                 // fused dc0 + sigmoid + assemble epilogue or nullptr
 };
 

@@ -13,6 +13,8 @@
 //     accumulators while reading the A tile from shared memory once;
 //   * in row-shared mode (full-resolution level, TW = W = 128) the A tile is a 130-voxel row (w halo, TMA zero fill)
 //     and the three kw taps are the same buffer shifted by one 128-byte row;
+//   * kh-shared mode swaps the roles of kh and kw: the M tile is a TH x TW sub-box placed anywhere in the slice, the
+//     A tile of one kw is a (TH + 2) x TW box and the three kh taps are the same buffer shifted by TW rows;
 //   * weights arrive as pre-swizzled blocks by cp.async.bulk and stay resident while the unit walks its input
 //     slices; the K loop can read two sources (decoder skip connection) so torch.cat is never materialised;
 //   * warp roles: 0 = TMA producer (activations), 1 = bulk producer (weights), 2 = MMA issuer + TMEM owner,
@@ -46,6 +48,12 @@ __device__ __forceinline__ BlockInfo decode_block(const ConvIgemmParams& p, int 
     bi.c = p.nkh == 3 ? b : b / 3;
     bi.kh = p.nkh == 3 ? 0 : b % 3;   // three-row stages start at row h - 1 and hold kh = 0, 1, 2
     bi.kw = 0;
+    bi.kdlo = 0;
+    bi.nkd = 3;
+  } else if (p.mode == kModeKhShared) {
+    bi.c = b / 3;
+    bi.kh = 0;   // the box starts at row h0 - 1 and holds kh = 0, 1, 2
+    bi.kw = b % 3;
     bi.kdlo = 0;
     bi.nkd = 3;
   } else if (p.mode == kModePerTap) {
@@ -84,8 +92,8 @@ struct UnitInfo {
 
 __device__ __forceinline__ UnitInfo decode_unit(const ConvIgemmParams& p, int u) {
   UnitInfo ui;
-  const int npw = p.W / p.TW;
-  const int np = npw * p.hp_cnt, ndg = (p.d_cnt + p.Rd - 1) / p.Rd;
+  const int npw = p.npw;
+  const int np = npw * p.nph, ndg = (p.d_cnt + p.Rd - 1) / p.Rd;
   if (p.w_stationary) {   // (N split, tap group) slowest: consecutive units of a CTA share their weight blocks
     const int per_key = np * ndg * p.NT;
     const int key = u / per_key;
@@ -102,8 +110,8 @@ __device__ __forceinline__ UnitInfo decode_unit(const ConvIgemmParams& p, int u)
   u /= np;
   ui.d0 = p.d_lo + (u % ndg) * p.Rd;
   ui.n = u / ndg;
-  ui.h0 = (p.hp_lo + patch / npw) * p.TH;
-  ui.w0 = (patch % npw) * p.TW;
+  ui.h0 = min(p.h_lo + (patch / npw) * p.TH, p.H - p.TH);   // the last tile of a range may overlap its neighbour
+  ui.w0 = min(p.w_lo + (patch % npw) * p.TW, p.W - p.TW);
   ui.rd = min(p.Rd, p.d_lo + p.d_cnt - ui.d0);
   ui.ra = (p.mode == kModeUp2) ? p.R : ui.rd;
   return ui;
@@ -281,7 +289,8 @@ __device__ __forceinline__ void mma_issuer_fast(const ConvIgemmParams& p, const 
   IssueConsts c;
   c.cout = static_cast<uint32_t>(p.cout);
   c.tap16 = (c.cout * rowb) >> 4;                               // one tap's weight rows, in descriptor units
-  c.kw_step = rowb >> 4;                                        // descriptor units per one-voxel row shift
+  // descriptor units between the taps of one A stage: one voxel row (row-shared kw), TW rows (kh-shared kh)
+  c.kw_step = (mode == kModeKhShared ? static_cast<uint32_t>(p.TW) * rowb : rowb) >> 4;
   c.desc_hi32 = (sbo >> 4) | (1u << 14) | (lay << 29);          // SBO, version = 1, swizzle mode
   c.idesc_1 = umma_idesc_f16(128, c.cout, p.ab_format);
   c.idesc_step = (c.cout >> 3) << 17;                           // +1 tap in the N field
@@ -396,7 +405,8 @@ __device__ __forceinline__ void mma_issuer_general(const ConvIgemmParams& p, con
                                                    uint64_t* acc_full, uint64_t* acc_empty) {
   const int mode = p.mode, R_acc = p.R, cout = p.cout, nblk = p.nblk, nst = p.n_astage, nwb = p.n_wbuf, Dm1 = p.D - 1,
             kpb = p.kd_per_block;
-  const int nkw = (mode == kModeRowShared) ? 3 : 1;
+  const int nkw = (mode == kModeRowShared || mode == kModeKhShared) ? 3 : 1;
+  const uint32_t a_tap = mode == kModeKhShared ? static_cast<uint32_t>(p.TW) * p.row_bytes : p.row_bytes;
   const int k16n = p.k16_steps;
   const uint32_t rowb = static_cast<uint32_t>(p.row_bytes), sbo = 8u * rowb, lay = rowb == 128u ? 2u : 4u;
   const uint32_t cout128 = static_cast<uint32_t>(cout) * rowb;    // bytes of one tap's weight rows
@@ -445,7 +455,7 @@ __device__ __forceinline__ void mma_issuer_general(const ConvIgemmParams& p, con
               tc_fence_after();
             }
             const uint32_t idesc = umma_idesc_f16(128, static_cast<uint32_t>(len * cout), p.ab_format);
-            const uint32_t a_addr = a_base + static_cast<uint32_t>(kw) * rowb;
+            const uint32_t a_addr = a_base + static_cast<uint32_t>(kw) * a_tap;
             const uint32_t b_addr = w_base + static_cast<uint32_t>(kw * ns + ti) * cout128;
             const uint32_t boff = p.base_off_mode ? ((a_addr >> 7) & 7u) : 0u;
             const uint32_t d_addr = tmem_base + static_cast<uint32_t>(a0 * cout);
@@ -598,7 +608,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
     // 1300 clocks for a lone warp -- against 6 x 96 clocks of MMAs for a 32-channel stage.  The loop body is therefore
     // specialised at compile time on (kw taps per stage, K=16 steps per chunk) and kept to descriptor adds.
     const bool general = p.base_off_mode || p.no_fast_path;
-    const int nkw_rt = (p.mode == kModeRowShared) ? 3 : 1;
+    const int nkw_rt = (p.mode == kModeRowShared || p.mode == kModeKhShared) ? 3 : 1;
     const int per_rt = max(1, 256 / p.cout);
 #define OAI_ISSUE(NKW, K16N, PER) \
   mma_issuer_fast<NKW, K16N, PER, 1>(p, tmem_base, abuf, wbuf, wstride, full_a, empty_a, full_w, empty_w, acc_full, acc_empty)

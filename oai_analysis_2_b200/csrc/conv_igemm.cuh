@@ -14,6 +14,8 @@ enum ConvMode : int {
   kModePointwise = 2,  // 1x1x1
   kModeUp2 = 3,        // ConvTranspose3d(k=2, s=2): the accumulators of a unit are sub-filters (taps) of ONE input
                        // M tile, stacked along N; the epilogue scatters each tap into the 2x output grid
+  kModeKhShared = 4,   // 3x3x3, M tile = TH x TW sub-box at any (h0, w0); one (TH+2) x TW box per kw, the kh taps are
+                       // the same buffer shifted by TW rows (a multiple of the 1024-byte swizzle atom)
 };
 
 // Optional fused epilogue of the last decoder layer: dc0 (1x1x1, C->ncls) + sigmoid (+ >0.5) + Partition.assemble
@@ -38,7 +40,8 @@ struct ConvIgemmParams {
   int up_groups;    // kModeUp2: tap groups per M tile (8 / R)
   long long tap_off[8];  // kModeUp2: output element offset of tap (a,b,c) = ((a*2H + b)*2W + c)*cout
   int d_lo, d_cnt;  // output region computed: slices [d_lo, d_lo+d_cnt) ...
-  int hp_lo, hp_cnt;  // ... and patch rows [hp_lo, hp_lo+hp_cnt) (units of TH voxel rows); the rest is dead halo
+  int h_lo, nph;     // ... and M tiles with origins (min(h_lo + i*TH, H-TH), min(w_lo + j*TW, W-TW)), i < nph, j < npw;
+  int w_lo, npw;    // the rest is dead halo
   int cout;         // N per accumulator (multiple of 16, <= 256)
   int nhalf;        // N splits (cout_total = nhalf*cout)
   int nchunks;      // K chunks (one TMA box of 64 channels each, 32 when row_bytes == 64) per tap set

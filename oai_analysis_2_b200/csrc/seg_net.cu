@@ -18,6 +18,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <set>
@@ -178,6 +179,12 @@ struct NamedTensor {
   long long numel;
 };
 
+// OAI_B200_SEG_W_HALO=0 keeps dc2 and dc1 in row-shared mode (whole 128-wide rows, the w halo computed and dropped)
+bool w_halo_skip_disabled() {
+  const char* e = getenv("OAI_B200_SEG_W_HALO");
+  return e && e[0] == '0';
+}
+
 int device_copy(const void* host, size_t bytes, void** dev) {
   if (int rc = check_cuda(cudaMalloc(dev, bytes), "seg_create: cudaMalloc")) return rc;
   return check_cuda(cudaMemcpy(*dev, host, bytes, cudaMemcpyHostToDevice), "seg_create: cudaMemcpy");
@@ -270,6 +277,9 @@ extern "C" int oai_seg_create(const oai_seg_config* cfg, const oai_tensor* state
     if (h->split[kPoolOf[i][1]]) h->split[kPoolOf[i][0]] = 1;
   needed_regions(h->tile, h->overlap, h->region);
   h->has_region = h->overlap[0] || h->overlap[1] || h->overlap[2];
+  // dc2 and dc1 (full resolution, 64 output channels) compute only their needed (h, w) box: kh-shared M tiles skip the
+  // dead w halo that row-shared tiles (one whole 128-wide row each) compute and throw away
+  const bool skip_w_halo = h->has_region && !w_halo_skip_disabled();
 
   // ---- consume the state dict (strict: every expected key present with the right shape, nothing left over)
   std::set<std::string> consumed;
@@ -337,7 +347,8 @@ extern "C" int oai_seg_create(const oai_seg_config* cfg, const oai_tensor* state
     s.kind = L.kind == 'u' ? 2 : 0;
     s.terms = h->terms[l];
     s.fmt = cfg->ab_format;
-    s.flags = 0;
+    // (where the tile is narrower than 128 these layers run per-tap tiles of whole rows, and stay so)
+    s.flags = (skip_w_halo && (l == DC2 || l == DC1) && s.W % 128 == 0) ? kConvFlagKhShared : 0;
     s.split0 = s.split1 = 0;   // filled per launch from the tensors actually bound
     ConvSpec ps = s;            // the packer only needs the terms' split pattern
     ps.split0 = s.terms == 2 || s.terms == 3 || s.terms == 5;
@@ -420,6 +431,21 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
   const int crop_zyx[3] = {h->cfg.overlap_xyz[2], h->cfg.overlap_xyz[0], h->cfg.overlap_xyz[1]};
   const int fmt = h->cfg.ab_format;
 
+  // a kh-shared launch over the w range [w_lo, w_hi]: 32-wide M tiles over the largest multiple of 32 columns, and a
+  // second launch of 8-wide tiles over the last columns when the width is not a multiple of 32 (dc2: 98 = 96 + 2, the
+  // strip covers the last 8 and overlaps the main tiles, which write the same values there)
+  auto conv_w_box = [&](const ConvSpec& s, ConvLaunch a, int w_lo, int w_hi) -> int {
+    const int w_cnt = w_hi - w_lo + 1, main = w_cnt / 32 * 32, rest = w_cnt - main;
+    if (main) {
+      a.w_lo = w_lo; a.w_cnt = main; a.flop_share = static_cast<double>(main) / w_cnt;
+      if (int rc = conv_run(s, a, st)) return rc;
+    }
+    if (!rest) return 0;
+    a.w_cnt = std::min((rest + 7) / 8 * 8, w_cnt);
+    a.w_lo = w_hi + 1 - a.w_cnt;
+    a.flop_share = static_cast<double>(rest) / w_cnt;   // the layer's algorithmic MACs are booked once
+    return conv_run(s, a, st);
+  };
   auto conv = [&](int l, int NT, int t0, int t1, int tout) -> int {
     const LayerDef& L = kLayers[l];
     const PackedLayer& P = h->layers[l];
@@ -448,6 +474,7 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
       a.region = region;
     }
     a.head = nullptr;
+    if (a.region && (s.flags & kConvFlagKhShared)) return conv_w_box(s, a, h->region[l].lo[2], h->region[l].hi[2]);
     return conv_run(s, a, st);
   };
   auto pool = [&](int i, int NT) -> int {
@@ -500,7 +527,7 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
     a.src0 = buf(T_D2); a.src1 = nullptr; a.NT = NT; a.wpack = P.w; a.wpack_bytes = P.w_bytes; a.bias = P.bias;
     a.relu = 1; a.out = nullptr; a.obase = a.osN = a.osD = a.osH = a.osW = 0; a.out_split = 0; a.out_lo_off = 0;
     a.region = region; a.head = &hd;
-    rc = conv_run(s, a, st);
+    rc = (s.flags & kConvFlagKhShared) ? conv_w_box(s, a, geom[8], geom[8] + geom[5] - 1) : conv_run(s, a, st);
   }
   nvtxRangePop();
   return rc;
