@@ -406,6 +406,28 @@ OAI_API int oai_surface_metrics(const uint8_t* mask_a, const uint8_t* mask_b, co
                                 const double* spacing_xyz, double* terms, long long* counts, float* dist_to_B,
                                 float* dist_to_A, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Connected components of a mask on dims = {D, H, W} (z, y, x): every axis at least 1 voxel and D*H*W < 2^31.
+ * connectivity 6, 18 or 26 is scipy.ndimage.generate_binary_structure(3, 1 / 2 / 3).  labels equal
+ * scipy.ndimage.label(mask, structure)[0] bit for bit: background 0, components 1..n in raster (C) order of their first
+ * voxel.  The workspace (256-byte aligned, oai_components_workspace_bytes(dims) bytes, 0 for unsupported dims) holds
+ * the rank map and the scan partials; the labels buffer doubles as the union-find parent array.  Integer results only
+ * (equal inputs give bitwise equal outputs); no host synchronisation, no allocation. */
+OAI_API size_t oai_components_workspace_bytes(const int* dims);
+/* Host-only upper bound on n, the length of the sizes buffer: ceil(D/2) ceil(H/2) ceil(W/2) for 26 (tight),
+ * ceil(D*H*W / 2) for 6 (tight: the checkerboard) and 18.  0 for unsupported dims or connectivity. */
+OAI_API long long oai_components_max(const int* dims, int connectivity);
+/* mask: device uint8 [dims], non-zero = inside; labels: device int32 [dims];
+ * sizes: device int32 [oai_components_max(dims, connectivity)], sizes[k - 1] = voxels of label k, zero past n;
+ * count: device int64, n. */
+OAI_API int oai_connected_components(const uint8_t* mask, const int* dims, int connectivity, int* labels, int* sizes,
+                                     long long* count, void* workspace, size_t workspace_bytes, void* stream);
+/* Keep policy on a labelled volume (labels, sizes, count of oai_connected_components): min_voxels < 0 keeps the largest
+ * component only (the lowest label on a tie, numpy's argmax), min_voxels >= 0 every component of at least min_voxels
+ * voxels.  The policy is read from the device-side sizes.  keep_mask (optional): device uint8 [dims], 1 = kept;
+ * values (optional): device float32 [dims], zeroed in place outside the kept components.  At least one is needed. */
+OAI_API int oai_keep_components(const int* labels, const int* sizes, const long long* count, const int* dims,
+                                int min_voxels, uint8_t* keep_mask, float* values, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------------
  * ITK-semantics warps  (reference: oai_analysis/dask_processing.py:95-111 deform_probmap_delayed,
  * test/test_all.py:42-52; transform = R_A o DisplacementFieldTransform o R_B^-1 built by create_itk_transform)

@@ -34,6 +34,8 @@ lib.oai_seg_workspace_bytes.restype = ctypes.c_size_t
 lib.oai_reg_workspace_bytes.restype = ctypes.c_size_t
 lib.oai_reg_loss_workspace_bytes.restype = ctypes.c_size_t
 lib.oai_seg_quality_workspace_bytes.restype = ctypes.c_size_t
+lib.oai_components_workspace_bytes.restype = ctypes.c_size_t
+lib.oai_components_max.restype = ctypes.c_longlong
 lib.oai_reg_convt4_umma_wbytes.restype = ctypes.c_size_t
 lib.oai_reg_conv3_umma_wbytes.restype = ctypes.c_size_t
 lib.oai_reg_conv3_umma_workspace.restype = ctypes.c_size_t

@@ -15,6 +15,11 @@ Checking a registration: warp knee A's segmentation onto knee B's grid, then com
     warped = (deform_probmap(phi_AB, image_A, image_B, fc_A, "FC"),
               deform_probmap(phi_AB, image_A, image_B, tc_A, "TC"))
     fc_q, tc_q = segmentation_metrics(warped, (fc_B, tc_B))
+
+How many pieces a mask falls into, and how much of its volume lies outside the main plate::
+
+    fc_c, tc_c = component_summary((fc, tc))
+    outside_mm3 = fc_c.total_mm3 - fc_c.largest_mm3
 """
 import collections
 
@@ -25,6 +30,7 @@ from . import itk_compat, ops
 
 SegmentationMetrics = collections.namedtuple("SegmentationMetrics",
                                              ["dice", "assd", "hd95", "hd", "volume_pred_mm3", "volume_ref_mm3"])
+ComponentSummary = collections.namedtuple("ComponentSummary", ["n_components", "largest_mm3", "total_mm3"])
 
 
 def _is_image(x):
@@ -60,6 +66,15 @@ def _mask(x, threshold):
     return t.contiguous() if t.dtype == torch.bool else t > threshold
 
 
+def _spacing(found, spacing_xyz):
+    spacing = found
+    if spacing is None:
+        if spacing_xyz is None:
+            raise ValueError("spacing_xyz is required for array or tensor inputs")
+        spacing = spacing_xyz
+    return tuple(float(v) for v in spacing)
+
+
 def segmentation_metrics(pred, ref, spacing_xyz=None, threshold=0.5):
     """Per-class quality of `pred` against `ref`: a list of SegmentationMetrics(dice, assd, hd95, hd, volume_pred_mm3,
     volume_ref_mm3), distances in mm.
@@ -75,12 +90,7 @@ def segmentation_metrics(pred, ref, spacing_xyz=None, threshold=0.5):
         raise ValueError(f"pred has {len(p_items)} classes and ref {len(r_items)}")
     if p_sp is not None and r_sp is not None and not np.allclose(p_sp, r_sp, rtol=1e-6, atol=0):
         raise ValueError(f"pred and ref grids differ in spacing: {p_sp} and {r_sp}")
-    spacing = p_sp or r_sp
-    if spacing is None:
-        if spacing_xyz is None:
-            raise ValueError("spacing_xyz is required for array or tensor inputs")
-        spacing = spacing_xyz
-    spacing = tuple(float(v) for v in spacing)
+    spacing = _spacing(p_sp or r_sp, spacing_xyz)
     voxel_mm3 = spacing[0] * spacing[1] * spacing[2]
     results = []
     for p, r in zip(p_items, r_items):
@@ -92,3 +102,18 @@ def segmentation_metrics(pred, ref, spacing_xyz=None, threshold=0.5):
     host = torch.stack([torch.cat([t, c.to(torch.float64)]) for t, c in results]).cpu().numpy()
     return [SegmentationMetrics(float(h[0]), float(h[1]), float(h[2]), float(h[3]), float(h[8]) * voxel_mm3,
                                 float(h[9]) * voxel_mm3) for h in host]
+
+
+def component_summary(pred, spacing_xyz=None, threshold=0.5, connectivity=6):
+    """Per-class connected components of `pred` (the inputs segmentation_metrics takes): a list of
+    ComponentSummary(n_components, largest_mm3, total_mm3), components as scipy.ndimage.label counts them with
+    connectivity 6, 18 or 26.  Synchronises once, to return Python numbers."""
+    items, sp = _classes(pred)
+    spacing = _spacing(sp, spacing_xyz)
+    voxel_mm3 = spacing[0] * spacing[1] * spacing[2]
+    rows = []
+    for p in items:
+        _, sizes, count = ops.connected_components(_mask(p, threshold), connectivity)
+        rows.append(torch.stack([count, sizes.max().to(torch.int64), sizes.sum(dtype=torch.int64)]))
+    host = torch.stack(rows).cpu().numpy()
+    return [ComponentSummary(int(h[0]), float(h[1]) * voxel_mm3, float(h[2]) * voxel_mm3) for h in host]

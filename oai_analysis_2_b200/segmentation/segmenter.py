@@ -41,7 +41,13 @@ class Segmenter3DInPatch(Segmenter):
         self.ready = False
 
     def pred_setup(self):
-        """segmenter.py:51-62."""
+        """segmenter.py:51-62.  Optional config key "keep_largest_component": 6, 18 or 26 makes segment_device zero
+        each class map outside the largest connected component (with that connectivity) of its > 0.5 mask; absent or
+        falsy leaves the output as the reference computes it."""
+        keep = self.config.get("keep_largest_component")
+        if keep and (isinstance(keep, bool) or keep not in (6, 18, 26)):
+            raise ValueError(f"keep_largest_component must be 6, 18 or 26 (a connectivity), got {keep!r}")
+        self.keep_largest = int(keep) if keep else None
         training_config = load_json_to_dict(self.config["training_config_file"])
         self.partition = Partition(training_config["patch_size"], self.config["overlap_size"],
                                    padding_mode="reflect", mode="pred")
@@ -71,8 +77,12 @@ class Segmenter3DInPatchClassWise(Segmenter3DInPatch):
         # mode); here the whole tile set is one batch unless the workspace would not fit the free device memory
         if tiles_per_batch is None:
             tiles_per_batch = self.config.get("tiles_per_batch") or handle.auto_tiles_per_batch(volume.shape)
-        return handle.forward(volume, out_mode=0 if if_output_prob_map else 1, tiles_per_batch=tiles_per_batch,
-                              out=out)
+        out = handle.forward(volume, out_mode=0 if if_output_prob_map else 1, tiles_per_batch=tiles_per_batch,
+                             out=out)
+        if self.keep_largest:
+            for c in range(out.shape[0]):
+                ops.keep_components(out[c], self.keep_largest)
+        return out
 
     def segment(self, image, if_output_prob_map=False, if_output_itk=True):
         if not self.ready:
