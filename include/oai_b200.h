@@ -114,6 +114,15 @@ OAI_API int oai_conv3d_igemm_ex(const void* src0, int c0, const void* src1, int 
                                 int W, const void* wpack, size_t wpack_bytes, const float* bias, int cout,
                                 int pointwise, int relu, int ab_format, int terms, void* out, int out_split, int flags,
                                 const int* region, void* stream);
+/* 8-bit lo planes: terms 6 / 7 are 4 / 2 (7 on one-source 3x3x3 layers only) with the split source stored as a plain
+ * 16-bit hi tensor (C channels, in_split = 0 for it) plus in_lo8, one e4m3 byte per channel and voxel holding
+ * satfinite(rn((x - hi) * 2^S)), S = 11 for fp16 and 8 for bf16; those chunks run as block-scaled 8-bit MMAs against
+ * e4m3 weights w * 2^T (T per layer, chosen at packing so that max|w| * 2^T <= 448).  out_lo8 (optional, out_split = 0)
+ * receives the output's lo plane in that format. */
+OAI_API int oai_conv3d_igemm_lo8(const void* src0, int c0, const void* src1, int c1, int in_split, const void* in_lo8,
+                                 int NT, int D, int H, int W, const void* wpack, size_t wpack_bytes, const float* bias,
+                                 int cout, int pointwise, int relu, int ab_format, int terms, void* out, int out_split,
+                                 void* out_lo8, int flags, const int* region, void* stream);
 
 /* fp16 saturation guard: how many epilogue threads of the conv kernel (on the current device, since the last reset) saw
  * an activation outside the fp16 range (|x| > 65504, or NaN) before rounding it.  Non-zero means the 16-bit tensors hold
@@ -164,7 +173,8 @@ OAI_API int oai_seg_head(const void* act, int C, int ncls, const float* w, const
  * ------------------------------------------------------------------------------------------------------------ */
 enum {
   OAI_SEG_PRECISION_FP16 = 0,    /* 16-bit operands everywhere (TF32-class mantissa, the reference's cuDNN default) */
-  OAI_SEG_PRECISION_MIXED = 1,   /* default: dc2's skip input (ec1's output) and dc1's input are read as fp16 hi+lo */
+  OAI_SEG_PRECISION_MIXED = 1,   /* default: dc2's skip input (ec1's output) and dc1's input are read as fp16 hi + e4m3
+                                  * lo (terms 6 / 7); OAI_B200_SEG_LO8=0 at oai_seg_create: fp16 hi+lo (terms 4 / 2) */
   OAI_SEG_PRECISION_FP16X2 = 2,  /* every layer reads fp16 hi+lo activations (terms 2) */
   OAI_SEG_PRECISION_FP16X3 = 3,  /* fp32-faithful: activations and weights both hi+lo (terms 3) */
   OAI_SEG_PRECISION_CUSTOM = 4   /* layer_terms[] below */
@@ -178,7 +188,8 @@ typedef struct {
   int precision;                          /* OAI_SEG_PRECISION_* */
   int layer_terms[17];                    /* CUSTOM only: terms of ec0..ec7, dc9..dc1 (ec0 is always exact): 1..3 as above;
                                            * 4 / 5 on a concatenating layer (dc8, dc5, dc2): only the skip / only the
-                                           * upsampled source is read as hi+lo */
+                                           * upsampled source is read as hi+lo; 6 on a concatenating layer: 4 with an e4m3
+                                           * lo plane; 7 on ec3, ec5, ec7, dc7, dc4 or dc1: 2 with an e4m3 lo plane */
 } oai_seg_config;
 
 /* one entry of the reference's state_dict: float32, contiguous, host memory, torch layout */

@@ -6,14 +6,16 @@
 
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
+#include <cuda_fp8.h>
 
+#include <cmath>
 #include <cstring>
 #include <vector>
 
 namespace oai {
 
-cudaError_t conv_igemm_launch(const ConvIgemmParams& p, const CUtensorMap& tm0, const CUtensorMap& tm1, int num_sms,
-                              cudaStream_t stream);
+cudaError_t conv_igemm_launch(const ConvIgemmParams& p, const CUtensorMap& tm0, const CUtensorMap& tm1,
+                              const CUtensorMap& tm2, int num_sms, cudaStream_t stream);
 cudaError_t conv_overflow_count(unsigned int* count, bool reset, cudaStream_t stream);
 
 namespace {
@@ -28,12 +30,13 @@ constexpr int kFlagNoPingPong = 128;  // A/B: k2s2 units use every TMEM column (
 constexpr int kFlagOneKhRow = 64;  // A/B: one kh row per A stage even where the three-row stage applies
 constexpr size_t kSmemBudget = 232448 - 1024 - 48 * 8 - 2112 - 2048;  // 227 KB minus alignment slack, barriers, head weights, bias
 
-// One K chunk of the implicit GEMM: a TMA box of 64 (32) channels starting at channel cc of source `src`.
+// One K chunk of the implicit GEMM: a TMA box of 64 (32) channels starting at channel cc of source `src` (kSrcLo8: the
+// e4m3 lo plane of input source `in`).
 // wsel picks the weight image multiplied with it: 0 = 16-bit weights rounded with error feedback, 1 = plain hi half,
-// 2 = lo half (w - hi); dup: the chunk runs over the [hi | lo] planes of a split tensor (virtual channel v < 2C maps
-// to input channel v mod C), otherwise over the first C channels only.
+// 2 = lo half (w - hi), 3 = e4m3(w * 2^T); dup: the chunk runs over the [hi | lo] planes of a split tensor (virtual
+// channel v < 2C maps to input channel v mod C), otherwise over the first C channels only.
 struct Chunk {
-  int src, cc, wsel, dup;
+  int src, cc, wsel, dup, in;
 };
 
 struct Plan {
@@ -50,6 +53,10 @@ struct Plan {
 inline bool split_src(int terms, int src) {
   return terms == 2 || terms == 3 || (terms == 4 && src == 1) || (terms == 5 && src == 0);
 }
+// which source a term code reads as a plain fp16 hi tensor plus an e4m3 lo plane: 6 the second (as 4), 7 the only one
+// (as 2 on a one-source layer)
+inline bool lo8_src(int terms, int src) { return (terms == 6 && src == 1) || (terms == 7 && src == 0); }
+inline bool lo8_terms(int terms) { return terms == 6 || terms == 7; }
 
 int build_chunks(const ConvSpec& s, Plan* pl) {
   int n = 0;
@@ -61,12 +68,17 @@ int build_chunks(const ConvSpec& s, Plan* pl) {
     const int wide = spl ? 2 * c : c;
     for (int j = 0; j * 64 < wide; ++j) {
       OAI_REQUIRE(n < kMaxChunks, "conv plan: more than %d K chunks", kMaxChunks);
-      pl->chunks[n++] = Chunk{src, j * 64, s.terms == 3 ? 1 : 0, spl ? 1 : 0};
+      pl->chunks[n++] = Chunk{src, j * 64, s.terms == 3 ? 1 : 0, spl ? 1 : 0, src};
     }
     if (s.terms == 3)
       for (int j = 0; j * 64 < c; ++j) {
         OAI_REQUIRE(n < kMaxChunks, "conv plan: more than %d K chunks", kMaxChunks);
-        pl->chunks[n++] = Chunk{src, j * 64, 2, 0};
+        pl->chunks[n++] = Chunk{src, j * 64, 2, 0, src};
+      }
+    if (lo8_src(s.terms, src))
+      for (int j = 0; j * 64 < c; ++j) {
+        OAI_REQUIRE(n < kMaxChunks, "conv plan: more than %d K chunks", kMaxChunks);
+        pl->chunks[n++] = Chunk{kSrcLo8, j * 64, 3, 0, src};
       }
   }
   pl->nch = n;
@@ -78,12 +90,15 @@ int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0, int tw = 32) {
   const int D = s.D, H = s.H, W = s.W, c0 = s.c0, c1 = s.c1, cout = s.cout, pointwise = s.kind, flags = s.flags;
   OAI_REQUIRE(D > 0 && H > 0 && W > 0 && c0 > 0 && c1 >= 0 && cout > 0, "conv plan: bad dims");
   OAI_REQUIRE(c0 % 8 == 0 && c1 % 8 == 0, "conv plan: channel counts must be multiples of 8 (got %d,%d)", c0, c1);
-  OAI_REQUIRE(s.terms >= 1 && s.terms <= 5,
+  OAI_REQUIRE(s.terms >= 1 && s.terms <= 7,
               "conv plan: terms=%d (1 = 16-bit, 2 = split activations, 3 = split both, 4 / 5 = split the second / first "
-              "source's activations only)", s.terms);
+              "source's activations only, 6 / 7 = 4 / 2 with an e4m3 lo plane)", s.terms);
   OAI_REQUIRE((!split_src(s.terms, 0) || s.split0) && (!split_src(s.terms, 1) || c1 == 0 || s.split1),
               "conv plan: terms=%d needs the split sources stored as [hi | lo] planes", s.terms);
-  OAI_REQUIRE(s.terms < 4 || c1 > 0, "conv plan: terms=%d is for two-source layers", s.terms);
+  OAI_REQUIRE(s.terms < 4 || s.terms > 6 || c1 > 0, "conv plan: terms=%d is for two-source layers", s.terms);
+  OAI_REQUIRE(s.terms != 7 || c1 == 0, "conv plan: terms=7 is for one-source layers");
+  OAI_REQUIRE(!lo8_terms(s.terms) || (pointwise == 0 && (s.terms == 6 ? c1 : c0) % 64 == 0),
+              "conv plan: terms=%d needs a 3x3x3 layer whose lo-plane source has a multiple of 64 channels", s.terms);
   OAI_REQUIRE((!s.split0 || c0 % 32 == 0) && (!s.split1 || c1 % 64 == 0) && (c1 == 0 || c0 % 64 == 0),
               "conv plan: split / concatenated sources need 64-channel multiples (got %d,%d)", c0, c1);
   pl->TW = W < 128 ? W : 128;
@@ -105,6 +120,14 @@ int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0, int tw = 32) {
   // as many accumulators as TMEM holds; the last d-group of a region may be partial
   int R = 512 / pl->cph < 8 ? 512 / pl->cph : 8;
   if (R > d_cnt) R = d_cnt;
+  if (lo8_terms(s.terms)) {
+    // the block scales of the e4m3 chunks take the TMEM columns from kSfaCol on; the d range is split into equal groups
+    // (dc2's 18 slices: 6 + 6 + 6 rather than 7 + 7 + 4)
+    const int rmax = kSfaCol / pl->cph < R ? kSfaCol / pl->cph : R;
+    OAI_REQUIRE(rmax >= 1, "conv plan: cout per split %d leaves no TMEM columns for the block scales", pl->cph);
+    const int groups = (d_cnt + rmax - 1) / rmax;
+    R = (d_cnt + groups - 1) / groups;
+  }
   pl->R = R;
   pl->Rd = R;
   pl->up_groups = 1;
@@ -193,9 +216,17 @@ int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0, int tw = 32) {
   return 0;
 }
 
-size_t plan_wpack_bytes(const Plan& pl) {
+bool plan_has_lo8(const Plan& pl) {
+  for (int c = 0; c < pl.nch; ++c)
+    if (pl.chunks[c].src == kSrcLo8) return true;
+  return false;
+}
+
+// the weight blocks, then (layers with lo8 chunks) 16 bytes holding the two UE8M0 block-scale words
+size_t plan_wblocks_bytes(const Plan& pl) {
   return static_cast<size_t>(pl.nhalf) * pl.up_groups * pl.nblk * pl.wblock_bytes;
 }
+size_t plan_wpack_bytes(const Plan& pl) { return plan_wblocks_bytes(pl) + (plan_has_lo8(pl) ? 16 : 0); }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -213,17 +244,21 @@ EncodeTiledFn encode_fn() {
   return fn;
 }
 
-// NDHWC 16-bit activation tensor viewed as a rank-5 TMA tensor (C, W, H, D, N); box = (64, bw, bh, 1, 1).
+// NDHWC activation tensor viewed as a rank-5 TMA tensor (C, W, H, D, N); box = (row_bytes of channels, bw, bh, 1, 1).
+// fmt: 0 fp16, 1 bf16, 2 one byte per channel (the e4m3 lo plane)
 int make_act_tmap(CUtensorMap* tm, const void* base, int C, int W, int H, int D, int N, int bw, int bh, int fmt,
                   int row_bytes = 128) {
   EncodeTiledFn fn = encode_fn();
   OAI_REQUIRE(fn != nullptr, "cuTensorMapEncodeTiled not available from the driver");
+  const cuuint64_t es = fmt == 2 ? 1 : 2;
   cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)N};
-  cuuint64_t strides[4] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2,
-                           (cuuint64_t)D * H * W * C * 2};
-  cuuint32_t box[5] = {(cuuint32_t)(row_bytes / 2), (cuuint32_t)bw, (cuuint32_t)bh, 1, 1};
+  cuuint64_t strides[4] = {(cuuint64_t)C * es, (cuuint64_t)W * C * es, (cuuint64_t)H * W * C * es,
+                           (cuuint64_t)D * H * W * C * es};
+  cuuint32_t box[5] = {(cuuint32_t)(row_bytes / es), (cuuint32_t)bw, (cuuint32_t)bh, 1, 1};
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = fn(tm, fmt == 0 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5,
+  const CUtensorMapDataType dt = fmt == 0 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                 : fmt == 1 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8;
+  CUresult r = fn(tm, dt, 5,
                   const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                   row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -251,6 +286,10 @@ inline size_t swz_off(int r, int j, int row_bytes) {
   const int chunk = j >> 3;
   const int sw = row_bytes == 128 ? (chunk ^ (r & 7)) : (chunk ^ ((r >> 1) & 3));
   return static_cast<size_t>(r) * row_bytes + (static_cast<size_t>(sw) << 4) + (j & 7) * 2;
+}
+// the same for byte element j of a 64-byte row (e4m3 rows, SWIZZLE_64B): 16 elements per 16-byte chunk
+inline size_t swz_off8(int r, int j) {
+  return static_cast<size_t>(r) * 64 + (static_cast<size_t>((j >> 4) ^ ((r >> 1) & 3)) << 4) + (j & 15);
 }
 
 inline float from16(uint16_t u, int fmt) {
@@ -326,6 +365,23 @@ int conv_pack_weights(const ConvSpec& s, const float* w, void* dst, size_t dst_b
     }
   }
   const int cs[2] = {s.c0, s.c1};
+  // e4m3 weights of the lo-plane chunks: w * 2^T with T the largest exponent that keeps max |w| * 2^T <= 448 (the
+  // e4m3 maximum) over the weights those chunks multiply
+  int T = 0;
+  const bool lo8 = plan_has_lo8(pl);
+  if (lo8) {
+    const int src = s.terms == 6 ? 1 : 0, ci0 = src == 0 ? 0 : s.c0;
+    float wmax = 0.f;
+    for (int co = 0; co < cout; ++co)
+      for (int ci = ci0; ci < ci0 + cs[src]; ++ci)
+        for (int t = 0; t < ktaps; ++t)
+          wmax = std::fmax(wmax, std::fabs(w[(static_cast<size_t>(co) * cin + ci) * ktaps + t]));
+    if (wmax > 0.f) T = static_cast<int>(std::floor(std::log2(448.0 / wmax)));
+    T = T < -100 ? -100 : (T > 100 ? 100 : T);
+    const int S = lo8_shift(fmt);
+    const uint32_t sf[2] = {static_cast<uint32_t>(127 - S) * 0x01010101u, static_cast<uint32_t>(127 - T) * 0x01010101u};
+    memcpy(out + plan_wblocks_bytes(pl), sf, sizeof(sf));
+  }
   const int ngroups = pl.up_groups;
   for (int nh = 0; nh < pl.nhalf; ++nh)
     for (int tg = 0; tg < ngroups; ++tg)
@@ -346,8 +402,8 @@ int conv_pack_weights(const ConvSpec& s, const float* w, void* dst, size_t dst_b
           c = b;
         }
         const Chunk& ck = pl.chunks[c];
-        const int csrc = cs[ck.src], cbase = ck.src == 0 ? 0 : s.c0;
-        const std::vector<uint16_t>& qq = q[ck.wsel];
+        const int csrc = cs[ck.in], cbase = ck.in == 0 ? 0 : s.c0;
+        const std::vector<uint16_t>& qq = q[ck.wsel == 3 ? 0 : ck.wsel];
         const int nstack = pl.mode == kModeUp2 ? pl.R : nkd;
         for (int kwi = 0; kwi < nkw; ++kwi)
           for (int ti = 0; ti < nstack; ++ti) {
@@ -359,6 +415,14 @@ int conv_pack_weights(const ConvSpec& s, const float* w, void* dst, size_t dst_b
             for (int co = 0; co < pl.cph; ++co) {
               const int r = (kwi * nstack + ti) * pl.cph + co;
               const uint16_t* wrow = qq.data() + (static_cast<size_t>(nh * pl.cph + co) * cin) * ktaps;
+              if (ck.wsel == 3) {
+                const float* wf = w + (static_cast<size_t>(nh * pl.cph + co) * cin) * ktaps;
+                for (int j = 0; j < 64 && ck.cc + j < csrc; ++j) {
+                  const float x = std::ldexp(wf[static_cast<size_t>(cbase + ck.cc + j) * ktaps + tap], T);
+                  blk[swz_off8(r, j)] = __nv_cvt_float_to_fp8(x, __NV_SATFINITE, __NV_E4M3);
+                }
+                continue;
+              }
               for (int j = 0; j < 64 && j * 2 < pl.row_bytes; ++j) {
                 const int v = ck.cc + j;
                 if (v >= (ck.dup ? 2 * csrc : csrc)) break;
@@ -416,6 +480,10 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
                   a.out_lo_off % 16 == 0 && (head || (reinterpret_cast<uintptr_t>(a.out) & 31) == 0),
               "conv: output base and strides must keep 32-byte alignment");
   OAI_REQUIRE(!(head && a.out_split), "conv head: the fused head writes class maps, not a split activation");
+  const bool lo8 = plan_has_lo8(pl);
+  OAI_REQUIRE(!lo8 || a.src_lo8, "conv: terms=%d reads an e4m3 lo plane; none given", s.terms);
+  OAI_REQUIRE(!a.out_lo8 || (!head && !a.out_split && (reinterpret_cast<uintptr_t>(a.out_lo8) & 31) == 0 && a.obase == 0),
+              "conv: an e4m3 lo output needs a plain 16-bit output at offset 0 and 32-byte alignment");
 
   ConvIgemmParams p;
   memset(&p, 0, sizeof(p));
@@ -441,6 +509,8 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
   p.out = a.out;
   p.obase = a.obase; p.osN = a.osN; p.osD = a.osD; p.osH = a.osH; p.osW = a.osW;
   p.out_split = a.out_split; p.out_lo_off = a.out_lo_off;
+  p.out_lo8 = static_cast<uint8_t*>(a.out_lo8);
+  p.lo8_sf_off = lo8 ? static_cast<uint32_t>(plan_wblocks_bytes(pl)) : 0u;
   p.d_lo = d_lo; p.d_cnt = d_cnt; p.h_lo = tile_h_lo; p.nph = nph; p.w_lo = kh_shared ? w_lo : 0; p.npw = npw;
   p.Rd = pl.Rd; p.up_groups = pl.up_groups;
   p.nunits = a.NT * ((d_cnt + pl.Rd - 1) / pl.Rd) * (nph * npw) * pl.up_groups * pl.nhalf;
@@ -455,12 +525,17 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
   OAI_REQUIRE(pl.mode != kModeUp2 || (c1 == 0 && !head), "conv: up2 mode takes one source and no fused head");
   const int bw = pl.mode == kModeRowShared ? 130 : pl.TW;
   const int bh = pl.mode == kModeKhShared ? pl.TH + 2 : pl.TH * pl.nkh;
-  CUtensorMap tm0, tm1;
+  CUtensorMap tm0, tm1, tm2;
   if (make_act_tmap(&tm0, a.src0, s.split0 ? 2 * c0 : c0, W, H, D, a.NT, bw, bh, s.fmt, pl.row_bytes)) return 1;
   if (a.src1) {
     if (make_act_tmap(&tm1, a.src1, s.split1 ? 2 * c1 : c1, W, H, D, a.NT, bw, bh, s.fmt)) return 1;
   } else {
     tm1 = tm0;
+  }
+  if (lo8) {
+    if (make_act_tmap(&tm2, a.src_lo8, s.terms == 6 ? c1 : c0, W, H, D, a.NT, bw, bh, 2, 64)) return 1;
+  } else {
+    tm2 = tm0;
   }
   ProfEntry* pe = nullptr;
   if (g_prof_on) {
@@ -478,7 +553,7 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
                      (static_cast<double>(pl.nch) * pl.k16 * 16);
     prof_record(pe->a, st);
   }
-  cudaError_t e = conv_igemm_launch(p, tm0, tm1, num_sms(), st);
+  cudaError_t e = conv_igemm_launch(p, tm0, tm1, tm2, num_sms(), st);
   if (pe) prof_record(pe->b, st);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   return check_cuda(e, "conv_igemm launch");
@@ -510,8 +585,8 @@ extern "C" int oai_conv3d_igemm_plan_ex(int D, int H, int W, int c0, int c1, int
   Plan pl;
   ConvSpec s = spec_of(D, H, W, c0, c1, cout, pointwise, 0, flags);
   s.terms = terms;
-  s.split0 = terms > 1;
-  s.split1 = terms > 1 && c1 > 0;
+  s.split0 = terms > 1 && !lo8_terms(terms);
+  s.split1 = terms > 1 && !lo8_terms(terms) && c1 > 0;
   if (make_plan(s, &pl)) return 1;
   plan[0] = pl.mode;
   plan[1] = pl.mode == kModeUp2 ? pl.up_groups : pl.kd_per_block;
@@ -535,8 +610,8 @@ extern "C" int oai_pack_conv_weights_ex(const float* w, int cout, int c0, int c1
                                         int terms, int ab_format, int flags, void* dst, size_t dst_bytes) {
   ConvSpec s = spec_of(D, H, W, c0, c1, cout, pointwise, ab_format, flags);
   s.terms = terms;
-  s.split0 = terms > 1;
-  s.split1 = terms > 1 && c1 > 0;
+  s.split0 = terms > 1 && !lo8_terms(terms);
+  s.split1 = terms > 1 && !lo8_terms(terms) && c1 > 0;
   return conv_pack_weights(s, w, dst, dst_bytes);
 }
 
@@ -576,6 +651,17 @@ extern "C" int oai_conv3d_igemm_ex(const void* src0, int c0, const void* src1, i
                                    int H, int W, const void* wpack, size_t wpack_bytes, const float* bias, int cout,
                                    int pointwise, int relu, int ab_format, int terms, void* out, int out_split,
                                    int flags, const int* region, void* stream) {
+  return oai_conv3d_igemm_lo8(src0, c0, src1, c1, in_split, nullptr, NT, D, H, W, wpack, wpack_bytes, bias, cout,
+                              pointwise, relu, ab_format, terms, out, out_split, nullptr, flags, region, stream);
+}
+
+// ... with e4m3 lo planes: in_lo8 is the lo plane of the source terms 6 / 7 read (one byte per channel and voxel),
+// out_lo8 (optional, with out_split = 0) receives the output's lo plane.
+extern "C" int oai_conv3d_igemm_lo8(const void* src0, int c0, const void* src1, int c1, int in_split,
+                                    const void* in_lo8, int NT, int D, int H, int W, const void* wpack,
+                                    size_t wpack_bytes, const float* bias, int cout, int pointwise, int relu,
+                                    int ab_format, int terms, void* out, int out_split, void* out_lo8, int flags,
+                                    const int* region, void* stream) {
   OAI_REQUIRE(out != nullptr, "conv: null output");
   OAI_REQUIRE(pointwise == 0 || pointwise == 1 || pointwise == 2, "conv: pointwise=%d", pointwise);
   ConvSpec s = spec_of(D, H, W, c0, c1, cout, pointwise, ab_format, flags);
@@ -586,6 +672,7 @@ extern "C" int oai_conv3d_igemm_ex(const void* src0, int c0, const void* src1, i
   ConvLaunch a;
   a.src0 = src0; a.src1 = src1; a.NT = NT; a.wpack = wpack; a.wpack_bytes = wpack_bytes; a.bias = bias; a.relu = relu;
   a.out = out; a.obase = 0; a.out_split = out_split; a.out_lo_off = cout; a.region = region; a.head = nullptr;
+  a.src_lo8 = in_lo8; a.out_lo8 = out_lo8;
   if (pointwise == 2) {
     a.osN = 8ll * D * H * W * cp; a.osD = 8ll * H * W * cp; a.osH = 4ll * W * cp; a.osW = 2 * cp;
   } else {

@@ -20,6 +20,8 @@ struct ConvSpec {
   int kind;            // 0 = 3x3x3 p1, 1 = 1x1x1, 2 = ConvTranspose3d(k2,s2)
   int terms;           // 1: a*w (16-bit operands) | 2: (a_hi + a_lo)*w | 3: a_hi*w_hi + a_lo*w_hi + a_hi*w_lo
                        // 4 / 5: as 2, but only source 1 / only source 0 is read as hi + lo
+                       // 6 / 7: as 4 / 2 (7: one-source layers), the source a plain fp16 hi tensor plus an e4m3 lo
+                       //        plane (ConvLaunch::src_lo8) multiplied by block-scaled 8-bit MMAs
   int fmt;             // 0 fp16, 1 bf16
   int flags;
 };
@@ -40,6 +42,8 @@ struct ConvLaunch {
   int w_lo = 0, w_cnt = 0;              // w range of the region (kConvFlagKhShared layers only; 0: full rows)
   double flop_share = 1.0;              // part of the layer's algorithmic MACs the profile books on this launch
   const HeadFuse* head;                 // fused dc0 + sigmoid + assemble epilogue or nullptr
+  const void* src_lo8 = nullptr;        // terms 6 / 7: e4m3 lo plane of the lo8 source (C bytes per voxel)
+  void* out_lo8 = nullptr;              // also write the output's e4m3 lo plane (cout bytes per voxel) here
 };
 
 size_t conv_wpack_bytes(const ConvSpec& s);

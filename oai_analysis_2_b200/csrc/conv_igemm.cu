@@ -145,12 +145,20 @@ __device__ __forceinline__ uint32_t pack2_residual(float a, float b, uint32_t hi
   return pack2<FMT>(a - h.x, b - h.y);
 }
 
+// rn(satfinite(e4m3)) of (a, b) scaled by 2^S, a in the low byte
+__device__ __forceinline__ uint32_t pack2_e4m3(float a, float b) {
+  uint16_t v;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(v) : "f"(b), "f"(a));
+  return v;
+}
+
 // Epilogue of one 32-column chunk held in registers: + bias (from shared memory), ReLU, 16-bit rounding, two 32-byte
-// stores per thread (a thread owns one voxel's channel row, so every L2 sector is written whole by one instruction);
-// SPLIT also writes the rounding residual lo = rn16(x - hi) lo_off elements further, so hi + lo carries ~22 bits.
-template <int FMT, bool RELU, bool SPLIT>
+// stores per thread (a thread owns one voxel's channel row, so every L2 sector is written whole by one instruction).
+// LO == 1 also writes the rounding residual lo = rn16(x - hi) lo_off elements further, so hi + lo carries ~22 bits;
+// LO == 2 writes it to the 8-bit plane dst8 instead, as e4m3(lo * 2^S) (one 32-byte store).
+template <int FMT, bool RELU, int LO>
 __device__ __forceinline__ void epi_store_chunk(uint32_t (&v)[32], uint32_t sbias, uint16_t* dst, long long lo_off,
-                                                float& amax) {
+                                                uint8_t* dst8, float& amax) {
   uint32_t o[16];
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
@@ -163,27 +171,47 @@ __device__ __forceinline__ void epi_store_chunk(uint32_t (&v)[32], uint32_t sbia
     amax = fmaxf(amax, fmaxf(fmaxf(fabsf(x0), fabsf(x1)), fmaxf(fabsf(x2), fabsf(x3))));
     o[2 * i] = pack2<FMT>(x0, x1);
     o[2 * i + 1] = pack2<FMT>(x2, x3);
-    if (SPLIT) {
+    if (LO) {
       v[4 * i] = __float_as_uint(x0); v[4 * i + 1] = __float_as_uint(x1);
       v[4 * i + 2] = __float_as_uint(x2); v[4 * i + 3] = __float_as_uint(x3);
     }
   }
   st_global_256(dst, o);
   st_global_256(dst + 16, o + 8);
-  if (SPLIT) {
+  if (LO == 1) {
 #pragma unroll
     for (int i = 0; i < 16; ++i)
       o[i] = pack2_residual<FMT>(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1]), o[i]);
     st_global_256(dst + lo_off, o);
     st_global_256(dst + lo_off + 16, o + 8);
+  } else if (LO == 2) {
+    constexpr float kScale = FMT == 0 ? 2048.f : 256.f;   // 2^lo8_shift(FMT)
+    uint32_t q[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      float2 h0, h1;
+      if (FMT == 0) {
+        h0 = __half22float2(*reinterpret_cast<const __half2*>(&o[2 * i]));
+        h1 = __half22float2(*reinterpret_cast<const __half2*>(&o[2 * i + 1]));
+      } else {
+        h0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&o[2 * i]));
+        h1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&o[2 * i + 1]));
+      }
+      const uint32_t lo01 = pack2_e4m3((__uint_as_float(v[4 * i]) - h0.x) * kScale,
+                                       (__uint_as_float(v[4 * i + 1]) - h0.y) * kScale);
+      const uint32_t lo23 = pack2_e4m3((__uint_as_float(v[4 * i + 2]) - h1.x) * kScale,
+                                       (__uint_as_float(v[4 * i + 3]) - h1.y) * kScale);
+      q[i] = lo01 | (lo23 << 16);
+    }
+    st_global_256(dst8, q);
   }
 }
 
 // All 32-column chunks of one accumulator (this warp's 32 TMEM lanes).  The accumulator is handed back to the MMA warp
 // as soon as its last columns sit in registers, before the conversion and the global stores of that batch.
-template <int FMT, bool RELU, bool SPLIT>
+template <int FMT, bool RELU, int LO>
 __device__ __forceinline__ void epi_store_acc(uint32_t t_acc, int nb, uint32_t sbias, uint16_t* dst, long long lo_off,
-                                              uint64_t* acc_empty_bar, int lane, float& amax) {
+                                              uint8_t* dst8, uint64_t* acc_empty_bar, int lane, float& amax) {
   for (int j = 0; j < nb; ++j) {
     uint32_t v[32];
     tmem_ld_32x32(t_acc + j * 32, v);
@@ -193,7 +221,7 @@ __device__ __forceinline__ void epi_store_acc(uint32_t t_acc, int nb, uint32_t s
       __syncwarp();
       if (lane == 0) mbar_arrive(acc_empty_bar);
     }
-    epi_store_chunk<FMT, RELU, SPLIT>(v, sbias + j * 128, dst + j * 32, lo_off, amax);
+    epi_store_chunk<FMT, RELU, LO>(v, sbias + j * 128, dst + j * 32, lo_off, dst8 + j * 32, amax);
   }
 }
 
@@ -231,11 +259,40 @@ __device__ __forceinline__ void head_dot(const uint32_t (&v)[32], uint32_t sbias
 struct IssueConsts {
   uint32_t kw_step, b_kw, desc_hi32, idesc_1, idesc_step, tap16, cout;
   uint32_t kh_a, kh_b;   // three-row stages: descriptor units between the kh rows of the A stage / the kh sub-blocks of B
+  uint32_t sfa, sfb;     // F8 stages: TMEM addresses of the block scales
 };
+
+// one MMA of a stage: kind::f16, or (F8) the block-scaled e4m3 kind with K = 32 over the same 32 bytes per row
+template <bool F8>
+__device__ __forceinline__ void issue_mma(const IssueConsts& c, uint32_t d, uint32_t a_lo, uint32_t b_lo, uint32_t idesc,
+                                          uint32_t acc) {
+  if (F8) umma_mxf8_ss_lohi(d, a_lo, b_lo, c.desc_hi32, idesc, c.sfa, c.sfb, acc);
+  else umma_f16_ss_lohi(d, a_lo, b_lo, c.desc_hi32, idesc, acc);
+}
+
+// shared-memory row pitch (128 or 64 bytes) and its K steps: every field of IssueConsts that depends on them
+__device__ __forceinline__ IssueConsts make_issue_consts(const ConvIgemmParams& p, uint32_t rowb, bool f8, int ns,
+                                                         uint32_t tmem_base) {
+  IssueConsts c;
+  const uint32_t sbo = 8u * rowb, lay = rowb == 128u ? 2u : 4u;
+  c.cout = static_cast<uint32_t>(p.cout);
+  c.tap16 = (c.cout * rowb) >> 4;                               // one tap's weight rows, in descriptor units
+  // descriptor units between the taps of one A stage: one voxel row (row-shared kw), TW rows (kh-shared kh)
+  c.kw_step = (p.mode == kModeKhShared ? static_cast<uint32_t>(p.TW) * rowb : rowb) >> 4;
+  c.desc_hi32 = (sbo >> 4) | (1u << 14) | (lay << 29);          // SBO, version = 1, swizzle mode
+  c.idesc_1 = f8 ? umma_idesc_mxf8_e4m3(128, c.cout) : umma_idesc_f16(128, c.cout, p.ab_format);
+  c.idesc_step = (c.cout >> 3) << 17;                           // +1 tap in the N field
+  c.b_kw = static_cast<uint32_t>(ns) * c.tap16;
+  c.kh_a = (130u * rowb) >> 4;
+  c.kh_b = 3u * c.b_kw;
+  c.sfa = tmem_base + kSfaCol;
+  c.sfb = tmem_base + kSfbCol;
+  return c;
+}
 
 // every (kw, k16) step of one A stage onto the accumulators [d_addr, +nt*cout), all accumulating; skip_first leaves out
 // the (0, 0) step (already issued by issue_first with per-accumulator overwrite flags)
-template <int NKW, int K16N, int PER, int NKH>
+template <int NKW, int K16N, int PER, int NKH, bool F8>
 __device__ __forceinline__ void issue_stage(const IssueConsts& c, uint32_t d_addr, uint32_t a_lo, uint32_t b_lo, int nt,
                                             bool skip_first) {
   for (int g0 = 0; g0 < nt; g0 += PER) {
@@ -250,10 +307,10 @@ __device__ __forceinline__ void issue_stage(const IssueConsts& c, uint32_t d_add
 #pragma unroll
         for (int k16 = 0; k16 < K16N; ++k16) {
           if (kh == 0 && kw == 0 && k16 == 0) {
-            if (!skip_first) umma_f16_ss_lohi(d, a_lo, bl, c.desc_hi32, idesc, 1u);
+            if (!skip_first) issue_mma<F8>(c, d, a_lo, bl, idesc, 1u);
           } else {
-            umma_f16_ss_lohi(d, a_lo + kh * c.kh_a + kw * c.kw_step + k16 * 2,
-                             bl + kh * c.kh_b + kw * c.b_kw + k16 * 2, c.desc_hi32, idesc, 1u);
+            issue_mma<F8>(c, d, a_lo + kh * c.kh_a + kw * c.kw_step + k16 * 2, bl + kh * c.kh_b + kw * c.b_kw + k16 * 2,
+                          idesc, 1u);
           }
         }
   }
@@ -261,7 +318,7 @@ __device__ __forceinline__ void issue_stage(const IssueConsts& c, uint32_t d_add
 
 // the (kw = 0, k16 = 0) step of a stage whose span [acc0, acc0 + nt) holds partial sums below accumulator f0 and is
 // fresh (first MMA of the unit: overwrite) from f0 on
-template <int PER>
+template <int PER, bool F8>
 __device__ __forceinline__ void issue_first(const IssueConsts& c, uint32_t tmem_base, int acc0, int nt, int f0,
                                             uint32_t a_lo, uint32_t b_lo) {
   for (int g0 = 0; g0 < nt; g0 += PER) {
@@ -270,30 +327,31 @@ __device__ __forceinline__ void issue_first(const IssueConsts& c, uint32_t tmem_
     const int keep = min(max(f0 - ag, 0), ng);  // leading accumulators of the group that accumulate
     const uint32_t bl = b_lo + static_cast<uint32_t>(g0) * c.tap16;
     if (keep > 0)
-      umma_f16_ss_lohi(tmem_base + static_cast<uint32_t>(ag) * c.cout, a_lo, bl, c.desc_hi32,
-                       c.idesc_1 + static_cast<uint32_t>(keep - 1) * c.idesc_step, 1u);
+      issue_mma<F8>(c, tmem_base + static_cast<uint32_t>(ag) * c.cout, a_lo, bl,
+                    c.idesc_1 + static_cast<uint32_t>(keep - 1) * c.idesc_step, 1u);
     if (keep < ng)
-      umma_f16_ss_lohi(tmem_base + static_cast<uint32_t>(ag + keep) * c.cout, a_lo,
-                       bl + static_cast<uint32_t>(keep) * c.tap16, c.desc_hi32,
-                       c.idesc_1 + static_cast<uint32_t>(ng - keep - 1) * c.idesc_step, 0u);
+      issue_mma<F8>(c, tmem_base + static_cast<uint32_t>(ag + keep) * c.cout, a_lo,
+                    bl + static_cast<uint32_t>(keep) * c.tap16,
+                    c.idesc_1 + static_cast<uint32_t>(ng - keep - 1) * c.idesc_step, 0u);
   }
 }
 
-template <int NKW, int K16N, int PER, int NKH>
+// chunk of weight block b (the block order of decode_block)
+__device__ __forceinline__ int block_chunk(const ConvIgemmParams& p, int b) {
+  if (p.mode == kModeRowShared) return p.nkh == 3 ? b : b / 3;
+  if (p.mode == kModeKhShared) return b / 3;
+  if (p.mode == kModePerTap) return p.kd_per_block == 3 ? b / 9 : b / 27;
+  return b;
+}
+
+// LO8: the layer lists e4m3 lo-plane chunks; their stages take the second, 8-bit form of the loop body (one uniform
+// branch per stage, block-scaled MMAs with K = 32, 64-byte rows)
+template <int NKW, int K16N, int PER, int NKH, bool LO8>
 __device__ __forceinline__ void mma_issuer_fast(const ConvIgemmParams& p, const uint32_t tmem_base0, uint8_t* abuf,
                                                 uint8_t* wbuf, const uint32_t wstride, uint64_t* full_a,
                                                 uint64_t* empty_a, uint64_t* full_w, uint64_t* empty_w,
                                                 uint64_t* acc_full0, uint64_t* acc_empty0) {
   const int mode = p.mode, R_acc = p.R, nblk = p.nblk, nst = p.n_astage, nwb = p.n_wbuf, Dm1 = p.D - 1;
-  const uint32_t rowb = static_cast<uint32_t>(p.row_bytes), sbo = 8u * rowb, lay = rowb == 128u ? 2u : 4u;
-  IssueConsts c;
-  c.cout = static_cast<uint32_t>(p.cout);
-  c.tap16 = (c.cout * rowb) >> 4;                               // one tap's weight rows, in descriptor units
-  // descriptor units between the taps of one A stage: one voxel row (row-shared kw), TW rows (kh-shared kh)
-  c.kw_step = (mode == kModeKhShared ? static_cast<uint32_t>(p.TW) * rowb : rowb) >> 4;
-  c.desc_hi32 = (sbo >> 4) | (1u << 14) | (lay << 29);          // SBO, version = 1, swizzle mode
-  c.idesc_1 = umma_idesc_f16(128, c.cout, p.ab_format);
-  c.idesc_step = (c.cout >> 3) << 17;                           // +1 tap in the N field
   const uint32_t a_lo0 = ((smem_u32(abuf) & 0x3FFFF) >> 4) | (1u << 16), a_step = p.astage_stride >> 4;
   const uint32_t w_lo0 = ((smem_u32(wbuf) & 0x3FFFF) >> 4) | (1u << 16), w_step = wstride >> 4;
   const bool up2 = mode == kModeUp2;
@@ -301,9 +359,8 @@ __device__ __forceinline__ void mma_issuer_fast(const ConvIgemmParams& p, const 
   const bool kd_cycle = mode == kModePerTap && p.kd_per_block == 1;
   const int ns = up2 ? R_acc : ((one_kd || kd_cycle) ? 1 : 3);  // taps stacked along N in every weight block
   const int a_inc = up2 ? 0 : 1;
-  c.b_kw = static_cast<uint32_t>(ns) * c.tap16;
-  c.kh_a = (130u * rowb) >> 4;
-  c.kh_b = 3u * c.b_kw;
+  const IssueConsts c = make_issue_consts(p, static_cast<uint32_t>(p.row_bytes), false, ns, tmem_base0);
+  const IssueConsts c8 = make_issue_consts(p, 64u, true, ns, tmem_base0);
   const bool stationary = p.w_stationary != 0;
   int prev_key = -1;
   const bool leader = elect_one();
@@ -344,6 +401,7 @@ __device__ __forceinline__ void mma_issuer_fast(const ConvIgemmParams& p, const 
       const int dhi = min(Dm1, d0 + rd - 1 + kdhi - 1);
       const bool last_blk = b == nblk - 1;
       if (reload) mbar_wait(&full_w[wb], wphase, 300 + wb);
+      const bool f8 = LO8 && p.chunk_src[block_chunk(p, b)] == kSrcLo8;
       const uint32_t w_lo = w_lo0 + static_cast<uint32_t>(wb) * w_step;
       int a_first = up2 ? 0 : dlo - kdhi + 1 - d0;  // accumulator hit by the first stacked tap
       for (int dp = dlo; dp <= dhi; ++dp, a_first += a_inc) {
@@ -353,7 +411,7 @@ __device__ __forceinline__ void mma_issuer_fast(const ConvIgemmParams& p, const 
         const int acc1 = min(a_first + ns - 1, ra - 1);
         const int nt = acc1 - acc0 + 1;
         const uint32_t d_addr = tmem_base + static_cast<uint32_t>(acc0) * c.cout;
-        const uint32_t b_lo = w_lo + static_cast<uint32_t>(acc0 - a_first) * c.tap16;
+        const uint32_t b_lo = w_lo + static_cast<uint32_t>(acc0 - a_first) * (f8 ? c8.tap16 : c.tap16);
         int f0 = -1;
         if (touched != all_acc) {
           // first weight block of the unit (and, in the one-kd schedule at the volume's first slice, the second):
@@ -369,8 +427,13 @@ __device__ __forceinline__ void mma_issuer_fast(const ConvIgemmParams& p, const 
         }
         const bool publish = last_blk && a_first >= 0 && a_first < ra;
         if (leader) {
-          if (f0 >= 0) issue_first<PER>(c, tmem_base, acc0, nt, f0, a_lo, b_lo);
-          issue_stage<NKW, K16N, PER, NKH>(c, d_addr, a_lo, b_lo, nt, f0 >= 0);
+          if (f8) {
+            if (f0 >= 0) issue_first<PER, true>(c8, tmem_base, acc0, nt, f0, a_lo, b_lo);
+            issue_stage<NKW, 2, PER, 1, true>(c8, d_addr, a_lo, b_lo, nt, f0 >= 0);
+          } else {
+            if (f0 >= 0) issue_first<PER, false>(c, tmem_base, acc0, nt, f0, a_lo, b_lo);
+            issue_stage<NKW, K16N, PER, NKH, false>(c, d_addr, a_lo, b_lo, nt, f0 >= 0);
+          }
           // release the A stage; the last block's last tap of an accumulator also publishes it to the epilogue
           umma_commit(&empty_a[stage]);
           if (publish) umma_commit(&acc_full[a_first]);
@@ -406,10 +469,6 @@ __device__ __forceinline__ void mma_issuer_general(const ConvIgemmParams& p, con
   const int mode = p.mode, R_acc = p.R, cout = p.cout, nblk = p.nblk, nst = p.n_astage, nwb = p.n_wbuf, Dm1 = p.D - 1,
             kpb = p.kd_per_block;
   const int nkw = (mode == kModeRowShared || mode == kModeKhShared) ? 3 : 1;
-  const uint32_t a_tap = mode == kModeKhShared ? static_cast<uint32_t>(p.TW) * p.row_bytes : p.row_bytes;
-  const int k16n = p.k16_steps;
-  const uint32_t rowb = static_cast<uint32_t>(p.row_bytes), sbo = 8u * rowb, lay = rowb == 128u ? 2u : 4u;
-  const uint32_t cout128 = static_cast<uint32_t>(cout) * rowb;    // bytes of one tap's weight rows
   const bool up2 = mode == kModeUp2;
   const bool leader = elect_one();
   int stage = 0, wb = 0;
@@ -421,6 +480,11 @@ __device__ __forceinline__ void mma_issuer_general(const ConvIgemmParams& p, con
     uint32_t touched = 0, signaled = 0;
     int kd_it = 0;  // kd counter of the one-kd-per-block schedule (fastest block index there)
     for (int b = 0; b < nblk; ++b) {
+      const bool f8 = p.chunk_src[block_chunk(p, b)] == kSrcLo8;   // e4m3 lo-plane chunk: 64-byte rows, K = 32 steps
+      const uint32_t rowb = f8 ? 64u : static_cast<uint32_t>(p.row_bytes), sbo = 8u * rowb, lay = rowb == 128u ? 2u : 4u;
+      const uint32_t a_tap = mode == kModeKhShared ? static_cast<uint32_t>(p.TW) * rowb : rowb;
+      const uint32_t cout128 = static_cast<uint32_t>(cout) * rowb;    // bytes of one tap's weight rows
+      const int k16n = f8 ? 2 : p.k16_steps;
       // taps stacked in this block and the input slices it walks (same arithmetic as decode_block, by counters)
       int kdlo = 0, nkd = 3;
       if (mode == kModePointwise || up2) { kdlo = 1; nkd = 1; }
@@ -454,7 +518,8 @@ __device__ __forceinline__ void mma_issuer_general(const ConvIgemmParams& p, con
                 mbar_wait(&acc_empty[a0 + j], ((use_bits >> (a0 + j)) & 1u) ^ 1u, 500 + a0 + j);
               tc_fence_after();
             }
-            const uint32_t idesc = umma_idesc_f16(128, static_cast<uint32_t>(len * cout), p.ab_format);
+            const uint32_t idesc = f8 ? umma_idesc_mxf8_e4m3(128, static_cast<uint32_t>(len * cout))
+                                      : umma_idesc_f16(128, static_cast<uint32_t>(len * cout), p.ab_format);
             const uint32_t a_addr = a_base + static_cast<uint32_t>(kw) * a_tap;
             const uint32_t b_addr = w_base + static_cast<uint32_t>(kw * ns + ti) * cout128;
             const uint32_t boff = p.base_off_mode ? ((a_addr >> 7) & 7u) : 0u;
@@ -463,7 +528,9 @@ __device__ __forceinline__ void mma_issuer_general(const ConvIgemmParams& p, con
               for (int k16 = 0; k16 < k16n; ++k16) {
                 const uint64_t adesc = umma_desc_kmajor(a_addr + k16 * 32, sbo, boff, lay);
                 const uint64_t bdesc = umma_desc_kmajor(b_addr + k16 * 32, sbo, 0, lay);
-                umma_f16_ss(d_addr, adesc, bdesc, idesc, (f | (k16 > 0)) ? 1u : 0u);
+                if (f8) umma_mxf8_ss(d_addr, adesc, bdesc, idesc, tmem_base + kSfaCol, tmem_base + kSfbCol,
+                                     (f | (k16 > 0)) ? 1u : 0u);
+                else umma_f16_ss(d_addr, adesc, bdesc, idesc, (f | (k16 > 0)) ? 1u : 0u);
               }
             }
             touched |= ((1u << len) - 1u) << a0;
@@ -501,7 +568,7 @@ __device__ __forceinline__ void mma_issuer_general(const ConvIgemmParams& p, con
 
 __global__ void __launch_bounds__(kThreads, 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant__ CUtensorMap tm1,
-                  const __grid_constant__ ConvIgemmParams p) {
+                  const __grid_constant__ CUtensorMap tm2, const __grid_constant__ ConvIgemmParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const uint32_t wstride = (p.wblock_bytes + 1023u) & ~1023u;
@@ -535,6 +602,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
     fence_mbar_init();
     tma_prefetch_desc(&tm0);
     tma_prefetch_desc(&tm1);
+    if (p.lo8_sf_off) tma_prefetch_desc(&tm2);
   }
   if (warp == 2) {
     tmem_alloc(tmem_slot, kTmemCols);
@@ -549,6 +617,20 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
+  if (p.lo8_sf_off) {
+    // block scales of the e4m3 chunks: every scale of A is 2^-S and every scale of B 2^-T, so whatever the hardware's
+    // scale-factor layout, two uniformly filled 32-column regions serve every MMA
+    if (warp >= 4 && warp < 8) {
+      const uint32_t* sf = reinterpret_cast<const uint32_t*>(p.wpack + p.lo8_sf_off);
+      const uint32_t lane_base = tmem_base + (static_cast<uint32_t>((warp & 3) * 32) << 16);
+      tmem_st_32x32_fill(lane_base + kSfaCol, __ldg(sf));
+      tmem_st_32x32_fill(lane_base + kSfbCol, __ldg(sf + 1));
+      tmem_st_wait();
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+  }
 
   if (warp == 0) {
     // ------------------------------------------------------------ activation producer
@@ -559,7 +641,9 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
         const UnitInfo ui = decode_unit(p, u);
         for (int b = 0; b < p.nblk; ++b) {
           const BlockInfo bi = decode_block(p, b);
-          const CUtensorMap* tm = p.chunk_src[bi.c] == 0 ? &tm0 : &tm1;
+          const int csrc = p.chunk_src[bi.c];
+          const CUtensorMap* tm = csrc == 0 ? &tm0 : csrc == 1 ? &tm1 : &tm2;
+          const uint32_t bytes = csrc == kSrcLo8 ? p.astage_bytes / 2 : p.astage_bytes;   // e4m3: 64-byte rows
           const int cc = p.chunk_cc[bi.c];
           const int kdhi = bi.kdlo + bi.nkd - 1;
           const int dlo = max(0, ui.d0 + bi.kdlo - 1);
@@ -568,7 +652,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
           const int ch = ui.h0 + bi.kh - 1;
           for (int dp = dlo; dp <= dhi; ++dp) {
             mbar_wait(&empty_a[stage], phase ^ 1u, 100 + stage);
-            mbar_arrive_expect_tx(&full_a[stage], p.astage_bytes);
+            mbar_arrive_expect_tx(&full_a[stage], bytes);
             tma_load_5d(abuf + static_cast<size_t>(stage) * p.astage_stride, tm, &full_a[stage], cc, cw, ch, dp, ui.n);
             if (++stage == p.n_astage) {
               stage = 0;
@@ -590,10 +674,12 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
         if (p.w_stationary && key == prev_key) continue;   // this group's blocks are still in shared memory
         prev_key = key;
         for (int b = 0; b < p.nblk; ++b) {
+          // the e4m3 rows of a lo-plane chunk fill the first half of its block
+          const uint32_t bytes = p.chunk_src[block_chunk(p, b)] == kSrcLo8 ? p.wblock_bytes / 2 : p.wblock_bytes;
           mbar_wait(&empty_w[wb], phase ^ 1u, 200 + wb);
-          mbar_arrive_expect_tx(&full_w[wb], p.wblock_bytes);
-          bulk_load(wbuf + static_cast<size_t>(wb) * wstride, src + static_cast<size_t>(b) * p.wblock_bytes,
-                    p.wblock_bytes, &full_w[wb]);
+          mbar_arrive_expect_tx(&full_w[wb], bytes);
+          bulk_load(wbuf + static_cast<size_t>(wb) * wstride, src + static_cast<size_t>(b) * p.wblock_bytes, bytes,
+                    &full_w[wb]);
           if (++wb == p.n_wbuf) {
             wb = 0;
             phase ^= 1u;
@@ -610,14 +696,21 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
     const bool general = p.base_off_mode || p.no_fast_path;
     const int nkw_rt = (p.mode == kModeRowShared || p.mode == kModeKhShared) ? 3 : 1;
     const int per_rt = max(1, 256 / p.cout);
-#define OAI_ISSUE(NKW, K16N, PER) \
-  mma_issuer_fast<NKW, K16N, PER, 1>(p, tmem_base, abuf, wbuf, wstride, full_a, empty_a, full_w, empty_w, acc_full, acc_empty)
+#define OAI_ISSUE_LO8(NKW, K16N, PER, LO8) \
+  mma_issuer_fast<NKW, K16N, PER, 1, LO8>(p, tmem_base, abuf, wbuf, wstride, full_a, empty_a, full_w, empty_w, acc_full, \
+                                          acc_empty)
+#define OAI_ISSUE(NKW, K16N, PER) OAI_ISSUE_LO8(NKW, K16N, PER, false)
 #define OAI_ISSUE_GENERAL() \
   mma_issuer_general(p, tmem_base, abuf, wbuf, wstride, full_a, empty_a, full_w, empty_w, acc_full, acc_empty)
+    const bool lo8 = p.lo8_sf_off != 0;
     if (general) OAI_ISSUE_GENERAL();
-    else if (nkw_rt == 3 && p.k16_steps == 4 && per_rt == 4) OAI_ISSUE(3, 4, 4);
+    else if (lo8) {
+      if (nkw_rt == 3 && p.k16_steps == 4 && per_rt == 4) OAI_ISSUE_LO8(3, 4, 4, true);
+      else if (nkw_rt == 1 && p.k16_steps == 4 && per_rt == 4) OAI_ISSUE_LO8(1, 4, 4, true);
+      else OAI_ISSUE_GENERAL();
+    } else if (nkw_rt == 3 && p.k16_steps == 4 && per_rt == 4) OAI_ISSUE(3, 4, 4);
     else if (nkw_rt == 3 && p.k16_steps == 2 && per_rt == 4 && p.nkh == 3)
-      mma_issuer_fast<3, 2, 4, 3>(p, tmem_base, abuf, wbuf, wstride, full_a, empty_a, full_w, empty_w, acc_full, acc_empty);
+      mma_issuer_fast<3, 2, 4, 3, false>(p, tmem_base, abuf, wbuf, wstride, full_a, empty_a, full_w, empty_w, acc_full, acc_empty);
     else if (nkw_rt == 3 && p.k16_steps == 2 && per_rt == 4) OAI_ISSUE(3, 2, 4);
     else if (nkw_rt == 1 && p.k16_steps == 4 && per_rt == 4) OAI_ISSUE(1, 4, 4);
     else if (nkw_rt == 1 && p.k16_steps == 4 && per_rt == 2) OAI_ISSUE(1, 4, 2);
@@ -625,11 +718,12 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
     else OAI_ISSUE_GENERAL();
 #undef OAI_ISSUE_GENERAL
 #undef OAI_ISSUE
+#undef OAI_ISSUE_LO8
   } else if (warp >= 4) {
     // ------------------------------------------------------------ epilogue
     const int q = warp & 3;                 // TMEM lane quadrant this warp may read
     const int eg = (warp - 4) >> 2;         // epilogue group: drains the accumulators a = eg, eg + kEpiGroups, ...
-    const int epi_variant = (p.ab_format ? 4 : 0) + (p.out_split ? 2 : 0) + (p.relu ? 1 : 0);
+    const int epi_variant = (p.ab_format ? 6 : 0) + (p.out_lo8 ? 4 : p.out_split ? 2 : 0) + (p.relu ? 1 : 0);
     const uint32_t s_bias_addr = smem_u32(s_bias), s_head_addr = smem_u32(s_head);
     const int m = q * 32 + lane;
     const int th = m / p.TW, tw = m % p.TW;
@@ -710,16 +804,24 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant
           const uint32_t sb = s_bias_addr + static_cast<uint32_t>(ui.nh * p.cout) * 4u;
           const uint32_t t_acc = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(a * p.cout);
           const int nb = p.cout / 32;
+          uint8_t* dst8 = p.out_lo8 + (dst - out);
+#define OAI_EPI(FMT, RELU, LO) \
+  epi_store_acc<FMT, RELU, LO>(t_acc, nb, sb, dst, p.out_lo_off, dst8, &acc_empty[a], lane, amax)
           switch (epi_variant) {
-            case 0: epi_store_acc<0, false, false>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
-            case 1: epi_store_acc<0, true, false>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
-            case 2: epi_store_acc<0, false, true>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
-            case 3: epi_store_acc<0, true, true>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
-            case 4: epi_store_acc<1, false, false>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
-            case 5: epi_store_acc<1, true, false>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
-            case 6: epi_store_acc<1, false, true>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
-            default: epi_store_acc<1, true, true>(t_acc, nb, sb, dst, p.out_lo_off, &acc_empty[a], lane, amax); break;
+            case 0: OAI_EPI(0, false, 0); break;
+            case 1: OAI_EPI(0, true, 0); break;
+            case 2: OAI_EPI(0, false, 1); break;
+            case 3: OAI_EPI(0, true, 1); break;
+            case 4: OAI_EPI(0, false, 2); break;
+            case 5: OAI_EPI(0, true, 2); break;
+            case 6: OAI_EPI(1, false, 0); break;
+            case 7: OAI_EPI(1, true, 0); break;
+            case 8: OAI_EPI(1, false, 1); break;
+            case 9: OAI_EPI(1, true, 1); break;
+            case 10: OAI_EPI(1, false, 2); break;
+            default: OAI_EPI(1, true, 2); break;
           }
+#undef OAI_EPI
           continue;  // accumulator already released
         }
         tc_fence_before();
@@ -756,8 +858,8 @@ cudaError_t conv_overflow_count(unsigned int* count, bool reset, cudaStream_t st
   return cudaMemcpyToSymbolAsync(g_fp16_overflow, &zero, sizeof(unsigned int), 0, cudaMemcpyHostToDevice, stream);
 }
 
-cudaError_t conv_igemm_launch(const ConvIgemmParams& p, const CUtensorMap& tm0, const CUtensorMap& tm1, int num_sms,
-                              cudaStream_t stream) {
+cudaError_t conv_igemm_launch(const ConvIgemmParams& p, const CUtensorMap& tm0, const CUtensorMap& tm1,
+                              const CUtensorMap& tm2, int num_sms, cudaStream_t stream) {
   const size_t smem = conv_igemm_smem_bytes(p);
   // the attribute is per device: cache what has been configured for each device of this process
   static size_t configured[64] = {0};
@@ -770,7 +872,7 @@ cudaError_t conv_igemm_launch(const ConvIgemmParams& p, const CUtensorMap& tm0, 
     if (dev >= 0 && dev < 64) configured[dev] = smem;
   }
   const int grid = p.nunits < num_sms ? p.nunits : num_sms;
-  conv_igemm_kernel<<<grid, kThreads, smem, stream>>>(tm0, tm1, p);
+  conv_igemm_kernel<<<grid, kThreads, smem, stream>>>(tm0, tm1, tm2, p);
   return cudaGetLastError();
 }
 

@@ -7,6 +7,14 @@
 namespace oai {
 
 constexpr int kMaxChunks = 48;
+constexpr int kSrcLo8 = 2;          // chunk_src value of a chunk read from the e4m3 lo plane (third tensor map)
+// TMEM columns of the block scales of a layer with lo8 chunks: SFA (activations) in [kSfaCol, +32), SFB (weights) in
+// [kSfbCol, +32); the accumulators of such a layer stay below kSfaCol
+constexpr int kSfaCol = 448;
+constexpr int kSfbCol = 480;
+// S: the lo plane holds (x - hi) * 2^S; |x - hi| <= 2^-11 |x| (fp16) or 2^-8 |x| (bf16), so lo * 2^S stays within the
+// e4m3 range (448) for |x| < 512
+inline constexpr int lo8_shift(int fmt) { return fmt == 0 ? 11 : 8; }
 
 enum ConvMode : int {
   kModeRowShared = 0,  // 3x3x3, M tile = one full 128-wide row; w halo loaded once, kw taps = smem row shifts
@@ -48,6 +56,8 @@ struct ConvIgemmParams {
   // chunk c reads channels [chunk_cc[c], +64) of tensor map chunk_src[c].  A plain layer lists source 0's channels then
   // source 1's (the decoder's torch.cat).  Split-precision layers (terms 2 / 3) read tensors stored as [hi | lo] fp16
   // planes (2C channels per voxel) and list more chunks: K-concatenation of a_hi*w, a_lo*w (and a_hi*w_lo).
+  // chunk_src == kSrcLo8 (terms 6 / 7): 64 channels of the e4m3 lo plane (64-byte rows, SWIZZLE_64B, half the bytes
+  // of a 16-bit chunk), multiplied with e4m3 weight rows by block-scaled 8-bit MMAs (K = 32).
   uint16_t chunk_cc[kMaxChunks];
   uint8_t chunk_src[kMaxChunks];
   int k16_steps;    // K=16 MMA steps per chunk: 4 (64 channels) or 2 (32 channels)
@@ -81,6 +91,12 @@ struct ConvIgemmParams {
   // split-precision consumers read); the os* strides then address the 2*C-channel voxel rows
   int out_split;
   long long out_lo_off;
+  // 8-bit lo output: a separate plane of one e4m3 byte per output element, satfinite(rn((x - hi) * 2^S)), S = lo8_shift(fmt),
+  // with the hi tensor's geometry (its byte offset equals the hi element offset); nullptr: none
+  uint8_t* out_lo8;
+  // layers with lo8 chunks: byte offset in wpack of the two UE8M0 scale words (2^-S for the activations, 2^-T for the
+  // weights, each byte of a word equal) the epilogue warps copy into the scale-factor columns of TMEM; 0: none
+  uint32_t lo8_sf_off;
   int nunits;
   HeadFuse head;
 };

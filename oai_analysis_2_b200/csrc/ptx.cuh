@@ -174,6 +174,36 @@ __device__ __forceinline__ void umma_f16_ss_lohi2(uint32_t tmem_d, uint32_t a_lo
       : "r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// Block-scaled 8-bit form: D[tmem] (+)= (A * SFA) * (B * SFB)^T with A, B e4m3 (K = 32 per instruction, 32 bytes per
+// row like a K = 16 fp16 step) and one UE8M0 scale per row and 32-wide K block read from TMEM at sfa / sfb.
+__device__ __forceinline__ void umma_mxf8_ss_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t desc_hi,
+                                                  uint32_t idesc, uint32_t tmem_sfa, uint32_t tmem_sfb,
+                                                  uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      ".reg .b64 da, db;\n\t"
+      "setp.ne.b32 p, %7, 0;\n\t"
+      "mov.b64 da, {%1, %3};\n\t"
+      "mov.b64 db, {%2, %3};\n\t"
+      "tcgen05.mma.cta_group::1.kind::mxf8f6f4.block_scale.scale_vec::1X [%0], da, db, %4, [%5], [%6], p;\n\t"
+      "}\n"
+      :
+      : "r"(tmem_d), "r"(a_lo), "r"(b_lo), "r"(desc_hi), "r"(idesc), "r"(tmem_sfa), "r"(tmem_sfb), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void umma_mxf8_ss(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                             uint32_t tmem_sfa, uint32_t tmem_sfb, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %6, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::mxf8f6f4.block_scale.scale_vec::1X [%0], %1, %2, %3, [%4], [%5], p;\n\t"
+      "}\n"
+      :
+      : "r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(tmem_sfa), "r"(tmem_sfb), "r"(accumulate)
+      : "memory");
+}
 // mbarrier arrive once every MMA issued so far by this thread has completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -201,6 +231,17 @@ __device__ __forceinline__ void tmem_ld_32x8(uint32_t taddr, uint32_t (&v)[8]) {
                : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// 32 lanes x 32 consecutive columns, every column of thread t's lane set to v
+__device__ __forceinline__ void tmem_st_32x32_fill(uint32_t taddr, uint32_t v) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+      "{%1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, "
+      "%1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1};"
+      :
+      : "r"(taddr), "r"(v)
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // Shared-memory matrix descriptor, K-major, 128-byte swizzle (rows of 128 B, 8-row groups `sbo_bytes` apart).
 // Field layout follows the sm_100 UMMA descriptor: [0,14) addr>>4, [16,30) LBO>>4, [32,46) SBO>>4,
@@ -229,6 +270,16 @@ __device__ __host__ __forceinline__ uint32_t umma_idesc_f16(uint32_t M, uint32_t
   d |= (ab_format & 7u) << 7;   // a_format
   d |= (ab_format & 7u) << 10;  // b_format
   d |= (N >> 3) << 17;
+  d |= (M >> 4) << 24;
+  return d;
+}
+
+// Instruction descriptor for kind::mxf8f6f4 with block scaling: A and B e4m3 (format 0), K-major, fp32 accumulate,
+// UE8M0 scale factors (bit 23), scale-factor byte 0 of A and B (bits [29,31) / [4,6)).
+__device__ __host__ __forceinline__ uint32_t umma_idesc_mxf8_e4m3(uint32_t M, uint32_t N) {
+  uint32_t d = 0;
+  d |= (N >> 3) << 17;
+  d |= 1u << 23;
   d |= (M >> 4) << 24;
   return d;
 }

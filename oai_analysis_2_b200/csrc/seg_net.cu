@@ -85,6 +85,7 @@ struct oai_seg_handle {
   int tile[3], overlap[3];   // z,y,x
   int terms[kNumLayers];
   int split[kNumTensors];
+  int lo8[kNumTensors];      // the tensor is a plain 16-bit hi tensor followed by an e4m3 lo plane (terms 6 / 7)
   PackedLayer layers[kNumLayers];
   float* stem_w = nullptr;   // [27][32]
   float* head_w = nullptr;   // [ncls][64]
@@ -97,11 +98,17 @@ namespace {
 
 int dims_at(const oai_seg_handle* h, int level, int a) { return h->tile[a] >> level; }
 
-size_t tensor_bytes(const oai_seg_handle* h, int t, int NT) {
+// bytes of the 16-bit part of a tensor ([hi | lo] planes when split); a lo8 tensor's e4m3 plane follows it
+size_t tensor_hi_bytes(const oai_seg_handle* h, int t, int NT) {
   const TensorDef& d = kTensors[t];
   size_t n = static_cast<size_t>(NT) * dims_at(h, d.level, 0) * dims_at(h, d.level, 1) * dims_at(h, d.level, 2) *
              d.channels * 2 * (h->split[t] ? 2 : 1);
   return (n + 255) & ~size_t(255);
+}
+
+size_t tensor_bytes(const oai_seg_handle* h, int t, int NT) {
+  const size_t hi = tensor_hi_bytes(h, t, NT);
+  return h->lo8[t] ? hi + (((hi / 2) + 255) & ~size_t(255)) : hi;   // 2 B + 1 B per channel and voxel
 }
 
 // First-fit offsets for the batch's activation tensors from their lifetimes; returns the peak.
@@ -185,6 +192,12 @@ bool w_halo_skip_disabled() {
   return e && e[0] == '0';
 }
 
+// OAI_B200_SEG_LO8=0 keeps the mixed plan's lo terms as fp16 planes (codes 4 / 2 instead of 6 / 7)
+bool lo8_disabled() {
+  const char* e = getenv("OAI_B200_SEG_LO8");
+  return e && e[0] == '0';
+}
+
 int device_copy(const void* host, size_t bytes, void** dev) {
   if (int rc = check_cuda(cudaMalloc(dev, bytes), "seg_create: cudaMalloc")) return rc;
   return check_cuda(cudaMemcpy(*dev, host, bytes, cudaMemcpyHostToDevice), "seg_create: cudaMemcpy");
@@ -216,8 +229,12 @@ extern "C" int oai_seg_layer_terms(int precision, int* terms17) {
     // of the network) 22; only its upsampled input 25; the skip input AND dc1's input 11; dc2 + dc1 entirely 5.
     // The default spends the split where it pays: dc2's skip source (code 4: 64 of its 192 input channels) and dc1
     // -- +9 ms per knee over all-fp16 instead of +20 ms for all of dc2, with fewer flips (min Dice 0.99932).
-    terms17[DC2] = 4;
-    terms17[DC1] = 2;
+    // The lo terms carry ~2^-11 of the activation, so they are stored as e4m3 planes and issued as block-scaled 8-bit
+    // MMAs at twice the fp16 rate (codes 6 / 7; adds ~2^-14 relative, 8x below the hi term's fp16 rounding);
+    // OAI_B200_SEG_LO8=0 keeps them as fp16 planes.
+    const bool lo8 = !lo8_disabled();
+    terms17[DC2] = lo8 ? 6 : 4;
+    terms17[DC1] = lo8 ? 7 : 2;
   } else if (precision == OAI_SEG_PRECISION_FP16X2 || precision == OAI_SEG_PRECISION_FP16X3) {
     for (int l = 1; l < kNumLayers; ++l) terms17[l] = precision == OAI_SEG_PRECISION_FP16X2 ? 2 : 3;
   }
@@ -259,7 +276,11 @@ extern "C" int oai_seg_create(const oai_seg_config* cfg, const oai_tensor* state
   if (cfg->precision == OAI_SEG_PRECISION_CUSTOM) {
     for (int l = 0; l < kNumLayers; ++l) {
       h->terms[l] = l == 0 ? 1 : cfg->layer_terms[l];
-      OAI_REQUIRE(h->terms[l] >= 1 && h->terms[l] <= 5 && (h->terms[l] < 4 || kLayers[l].c_first > 0),
+      const int tm = h->terms[l];
+      // 4 / 5 / 6 on concatenating layers only; 7 on one-source 3x3x3 layers whose input a conv writes
+      const bool conv_input = l == EC3 || l == EC5 || l == EC7 || l == DC7 || l == DC4 || l == DC1;
+      OAI_REQUIRE(tm >= 1 && tm <= 7 && ((tm != 4 && tm != 5 && tm != 6) || kLayers[l].c_first > 0) &&
+                      (tm != 7 || conv_input),
                   "seg_create: layer_terms[%d]=%d", l, h->terms[l]);
     }
   } else if (oai_seg_layer_terms(cfg->precision, h->terms)) {
@@ -272,9 +293,15 @@ extern "C" int oai_seg_create(const oai_seg_config* cfg, const oai_tensor* state
     const bool is_skip = t == T_SYN0 || t == T_SYN1 || t == T_SYN2;
     const int tm = c >= 0 ? h->terms[c] : 1;
     h->split[t] = tm == 2 || tm == 3 || (tm == 4 && is_skip) || (tm == 5 && !is_skip);
+    h->lo8[t] = (tm == 6 && is_skip) || tm == 7;
   }
-  for (int i = 0; i < 3; ++i)   // a skip tensor must also carry both planes when its pooled consumer wants them
+  for (int i = 0; i < 3; ++i) {  // a skip tensor must also carry both planes when its pooled consumer wants them
     if (h->split[kPoolOf[i][1]]) h->split[kPoolOf[i][0]] = 1;
+    // the pool reads the 16-bit part only, so a lo8 skip tensor pools like a plain one; a skip tensor cannot be both
+    OAI_REQUIRE(!(h->split[kPoolOf[i][0]] && h->lo8[kPoolOf[i][0]]),
+                "seg_create: layer_terms: %s reads its skip input with an e4m3 lo plane while %s needs it as fp16 hi + lo",
+                kLayers[kTensors[kPoolOf[i][0]].consumers[0]].name, kLayers[kPoolOf[i][2]].name);
+  }
   needed_regions(h->tile, h->overlap, h->region);
   h->has_region = h->overlap[0] || h->overlap[1] || h->overlap[2];
   // dc2 and dc1 (full resolution, 64 output channels) compute only their needed (h, w) box: kh-shared M tiles skip the
@@ -350,7 +377,7 @@ extern "C" int oai_seg_create(const oai_seg_config* cfg, const oai_tensor* state
     // (where the tile is narrower than 128 these layers run per-tap tiles of whole rows, and stay so)
     s.flags = (skip_w_halo && (l == DC2 || l == DC1) && s.W % 128 == 0) ? kConvFlagKhShared : 0;
     s.split0 = s.split1 = 0;   // filled per launch from the tensors actually bound
-    ConvSpec ps = s;            // the packer only needs the terms' split pattern
+    ConvSpec ps = s;            // the packer only needs the terms' split pattern (lo8 sources are plain hi tensors)
     ps.split0 = s.terms == 2 || s.terms == 3 || s.terms == 5;
     ps.split1 = (s.terms == 2 || s.terms == 3 || s.terms == 4) && s.c1 > 0;
     P.w_bytes = conv_wpack_bytes(ps);
@@ -425,6 +452,7 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
               workspace_bytes, nb, need);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   auto buf = [&](int t) { return static_cast<void*>(ws + offs[t]); };
+  auto lo8buf = [&](int t) { return h->lo8[t] ? static_cast<void*>(ws + offs[t] + tensor_hi_bytes(h, t, nb)) : nullptr; };
   const int geom[12] = {h->tile[0], h->tile[1], h->tile[2], eff[0], eff[1], eff[2],
                         h->overlap[0], h->overlap[1], h->overlap[2], grid[0], grid[1], grid[2]};
   // assemble's crop_size indexing: crop_size (x,y,z) is read as [2], [0], [1] for z, y, x (image_transforms.py:511)
@@ -457,6 +485,8 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
     a.src1 = t1 >= 0 ? buf(t1) : nullptr;
     a.NT = NT; a.wpack = P.w; a.wpack_bytes = P.w_bytes; a.bias = P.bias; a.relu = 1;
     a.out = buf(tout);
+    a.out_lo8 = lo8buf(tout);
+    a.src_lo8 = lo8buf(s.terms == 6 ? t1 : t0);
     a.obase = 0;
     a.out_split = h->split[tout];
     a.out_lo_off = L.cout;
@@ -526,7 +556,7 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
     ConvLaunch a;
     a.src0 = buf(T_D2); a.src1 = nullptr; a.NT = NT; a.wpack = P.w; a.wpack_bytes = P.w_bytes; a.bias = P.bias;
     a.relu = 1; a.out = nullptr; a.obase = a.osN = a.osD = a.osH = a.osW = 0; a.out_split = 0; a.out_lo_off = 0;
-    a.region = region; a.head = &hd;
+    a.region = region; a.head = &hd; a.src_lo8 = lo8buf(T_D2);
     rc = (s.flags & kConvFlagKhShared) ? conv_w_box(s, a, geom[8], geom[8] + geom[5] - 1) : conv_run(s, a, st);
   }
   nvtxRangePop();

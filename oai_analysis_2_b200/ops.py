@@ -207,6 +207,22 @@ def split16(x, ab_format=0):
     return torch.cat((hi, lo), dim=-1).contiguous()
 
 
+LO8_SHIFT = (11, 8)   # S per 16-bit format: the e4m3 lo plane holds (x - hi) * 2^S
+
+
+def split_lo8(x, ab_format=0):
+    """float32 [..., C] -> (hi [..., C] 16-bit, lo8 [..., C] uint8): hi = rn16(x) and the e4m3 bytes of
+    satfinite(rn((x - hi) * 2^S)) -- the layout terms 6 / 7 read."""
+    hi = x.to(_DT16[ab_format])
+    lo = ((x - hi.float()) * 2.0 ** LO8_SHIFT[ab_format]).clamp(-448.0, 448.0)
+    return hi.contiguous(), lo.to(torch.float8_e4m3fn).view(torch.uint8).contiguous()
+
+
+def lo8_value(lo8, ab_format=0):
+    """uint8 e4m3 plane -> float32 x - hi it stands for."""
+    return lo8.view(torch.float8_e4m3fn).float() * 2.0 ** -LO8_SHIFT[ab_format]
+
+
 def conv_plan_ex(D, H, W, c0, c1, cout, pointwise=0, terms=1, flags=0):
     plan = (c_int * 10)()
     check(lib.oai_conv3d_igemm_plan_ex(D, H, W, c0, c1, cout, int(pointwise), int(terms), flags, plan), "conv plan")
@@ -228,19 +244,23 @@ def pack_conv_weights_ex(w, c0, c1, D, H, W, pointwise=0, terms=1, ab_format=0, 
 
 
 def conv3d_igemm_ex(src0, src1, wpack, bias, cout, c0, c1=0, pointwise=0, relu=True, ab_format=0, terms=1,
-                    in_split=False, out_split=False, region=None, flags=0):
-    """Split-precision form of conv3d_igemm: src* are [NT,D,H,W,C] (or [.., 2C] = [hi | lo] when in_split)."""
+                    in_split=False, out_split=False, region=None, flags=0, in_lo8=None, out_lo8=False):
+    """Split-precision form of conv3d_igemm: src* are [NT,D,H,W,C] (or [.., 2C] = [hi | lo] when in_split).
+    terms 6 / 7: in_lo8 is the uint8 e4m3 lo plane of the split source (split_lo8); out_lo8: also return the output's
+    lo plane, (out, lo8)."""
     NT, D, H, W, _ = src0.shape
     assert src0.is_contiguous() and (src1 is None or src1.is_contiguous())
+    assert in_lo8 is None or (in_lo8.dtype == torch.uint8 and in_lo8.is_contiguous())
     up = 2 if pointwise == 2 else 1
     out = torch.empty((NT, up * D, up * H, up * W, cout * (2 if out_split else 1)), dtype=_DT16[ab_format],
                       device=src0.device)
+    lo8 = torch.empty(out.shape, dtype=torch.uint8, device=src0.device) if out_lo8 else None
     reg = None if region is None else np.asarray(region, dtype=np.int32)
-    check(lib.oai_conv3d_igemm_ex(ptr(src0), c0, ptr(src1), c1, int(in_split), NT, D, H, W, ptr(wpack),
-                                  c_size(wpack.numel()), ptr(bias), cout, int(pointwise), int(relu), ab_format,
-                                  int(terms), ptr(out), int(out_split), flags, ptr(reg), stream_ptr()),
+    check(lib.oai_conv3d_igemm_lo8(ptr(src0), c0, ptr(src1), c1, int(in_split), ptr(in_lo8), NT, D, H, W, ptr(wpack),
+                                   c_size(wpack.numel()), ptr(bias), cout, int(pointwise), int(relu), ab_format,
+                                   int(terms), ptr(out), int(out_split), ptr(lo8), flags, ptr(reg), stream_ptr()),
           "conv3d_igemm_ex")
-    return out
+    return (out, lo8) if out_lo8 else out
 
 
 def seg_head(act, w, b, out, geom, tile0, crop_zyx, out_mode=0, ab_format=0):

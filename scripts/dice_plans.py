@@ -19,6 +19,7 @@ def main():
              "dc2", "dc1"]
     plans = {"fp16": {}, "dc2 (mixed)": {"dc2": 2}, "dc1+dc2": {"dc1": 2, "dc2": 2},
              "dc2 skip only": {"dc2": 4}, "dc2 skip + dc1": {"dc2": 4, "dc1": 2}, "dc2 up only": {"dc2": 5},
+             "dc2 skip + dc1 lo8 (mixed)": {"dc2": 6, "dc1": 7},
              "dc2 skip + dc1 x3": {"dc2": 4, "dc1": 3}, "dc2 skip + dc1 + ec1": {"dc2": 4, "dc1": 2, "ec1": 2},
              "dc2 skip + dc1 + dc5 skip": {"dc2": 4, "dc1": 2, "dc5": 4}, "dc2 up + dc1": {"dc2": 5, "dc1": 2},
              "dc2 skip + dc1 + ec2": {"dc2": 4, "dc1": 2, "ec2": 2},

@@ -5,7 +5,8 @@ north-star Dice >= 0.999 bar?  (Design aid for the conv kernel's precision modes
 
 Each layer's (BN-folded) weights and stored activations are rounded the way a candidate kernel mode would round
 them; products/accumulation are fp32 like the tensor pipe.  Modes per layer: w in {"h" fp16 error-feedback,
-"hl" fp16 hi+lo}, a (the layer's INPUT activation) in {"h", "hl"}.
+"hl" fp16 hi+lo}, a (the layer's INPUT activation) in {"h", "hl", "l8" fp16 hi + e4m3 lo plane (terms 6 / 7; the
+e4m3 rounding of the weights the lo plane meets is left out: it scales a term already 2^-11 of the activation)}.
 """
 import os
 import sys
@@ -48,6 +49,13 @@ def q_hl(x):
     return hi + q16(x - hi)
 
 
+def q_l8(x):
+    """fp16 hi + the e4m3 lo plane: satfinite(rn((x - hi) * 2^11)) * 2^-11"""
+    hi = q16(x)
+    lo = ((x - hi) * 2.0 ** 11).clamp(-448.0, 448.0).to(torch.float8_e4m3fn).to(x.dtype)
+    return hi + lo * 2.0 ** -11
+
+
 def q_w_ef(w):
     """error feedback along the taps of each (co, ci) filter, as oai_pack_conv_weights does"""
     co, ci = w.shape[:2]
@@ -88,6 +96,8 @@ def run(name, plan, act_default="h", verbose=True):
             return x
         if "hl" in consumer_modes:
             return q_hl(x)
+        if "l8" in consumer_modes:
+            return q_l8(x)
         return q16(x)
 
     am = lambda n: plan.get(n, ("h", act_default))[1]  # noqa: E731
@@ -127,8 +137,9 @@ def run(name, plan, act_default="h", verbose=True):
     tc = so.assemble(pred[:, 1].numpy(), g, m["overlap"])
     e = max(np.abs(fc - z["fc"]).max(), np.abs(tc - z["tc"]).max())
     d_fc, d_tc = dice(fc, z["fc_mask"]), dice(tc, z["tc_mask"])
+    flips = int(((fc > 0.5) != z["fc_mask"]).sum() + ((tc > 0.5) != z["tc_mask"]).sum())
     if verbose:
-        print(f"{name}: max-abs {e:.2e}  Dice FC {d_fc:.5f} TC {d_tc:.5f}")
+        print(f"{name}: max-abs {e:.2e}  Dice FC {d_fc:.5f} TC {d_tc:.5f}  mask flips {flips}")
     return e, d_fc, d_tc
 
 
@@ -145,3 +156,7 @@ if __name__ == "__main__":
     run(name, {n: ("h", "hl") for n in LAYERS})
     print("both hi+lo (3-term):")
     run(name, {n: ("hl", "hl") for n in LAYERS})
+    print("mixed with fp16 lo planes (dc2's skip input and dc1's input hi+lo, codes 4 / 2):")
+    run(name, {"dc2.skip": ("h", "hl"), "dc1": ("h", "hl")})
+    print("mixed with e4m3 lo planes (codes 6 / 7, the default):")
+    run(name, {"dc2.skip": ("h", "l8"), "dc1": ("h", "l8")})
