@@ -57,7 +57,15 @@ OAI_API int oai_conv3d_igemm(const void* src0, int c0, const void* src1, int c1,
 /* oai_conv3d_igemm restricted to the output sub-box region = {d_lo, d_cnt, h_lo, h_cnt} (full rows in w).  The
  * reference computes every decoder layer on the whole tile and then keeps only the tile interior
  * (image_transforms.py:497-503); outputs no kept voxel depends on ("dead halo") need not be computed.  Results inside
- * the region are identical to the full-layer call; memory outside it is left untouched. */
+ * the region are identical to the full-layer call.  The kernel computes whole M tiles, so voxels of the d range outside
+ * [h_lo, h_lo + h_cnt) may be written too, always with their full-layer values:
+ *   - row-shared / per-tap / pointwise / k2s2 layers: every row of the TH-row tiles the region's rows fall in, tiles
+ *     aligned to multiples of TH = 128 / min(W, 128) (k2s2: on the input grid, the written set is its 2x image);
+ *   - kh-shared layers: TH = 128 / tw rows per tile, tw in {32, 16, 8} the width with the fewest tiles over the
+ *     h_cnt x W box (the widest on a tie); tiles start at h_lo, h_lo + TH, ... and each is clamped to start at most at
+ *     H - TH, so the written rows are [min(h_lo, H - TH), min(h_lo + ceil(h_cnt / TH) * TH, H)).
+ * Slices outside [d_lo, d_lo + d_cnt) are left untouched.
+ * tests/test_conv_conformance_gpu.py pins this down. */
 OAI_API int oai_conv3d_igemm_region(const void* src0, int c0, const void* src1, int c1, int NT, int D, int H, int W,
                                     const void* wpack, size_t wpack_bytes, const float* bias, int cout, int pointwise,
                                     int relu, int ab_format, void* out, long long obase, long long osN, long long osD,
@@ -78,7 +86,8 @@ OAI_API int oai_convt2_igemm(const void* src, int cin, int NT, int D, int H, int
  * (networks.py:64) feeding dc0 = Conv3d(64->ncls,k1) (networks.py:66,148), torch.sigmoid (segmenter.py:121)
  * [out_mode 1: ">0.5", segmenter.py:123-124; 2: raw logits] and Partition.assemble's crop-and-place with the zeroed
  * border shell (image_transforms.py:492-513).  dc0 is evaluated on the fp32 accumulators, the 64-channel activation is
- * never written.  out: float32 [ncls][vol_dims]; geom / vol_dims / crop_zyx as for oai_seg_head. */
+ * never written.  out: float32 [ncls][vol_dims]; geom / vol_dims / crop_zyx as for oai_seg_head.  Only the tile
+ * interior is computed; with the kh-shared flag (256) its (h, w) box runs as oai_conv3d_igemm_box does. */
 OAI_API int oai_conv3d_igemm_head(const void* src0, int c0, const void* src1, int c1, int NT, int D, int H, int W,
                                   const void* wpack, size_t wpack_bytes, const float* bias, int ab_format, int ncls,
                                   const float* head_w, const float* head_b, float* out, const int* vol_dims,
@@ -123,6 +132,15 @@ OAI_API int oai_conv3d_igemm_lo8(const void* src0, int c0, const void* src1, int
                                  int NT, int D, int H, int W, const void* wpack, size_t wpack_bytes, const float* bias,
                                  int cout, int pointwise, int relu, int ab_format, int terms, void* out, int out_split,
                                  void* out_lo8, int flags, const int* region, void* stream);
+/* oai_conv3d_igemm_lo8 (3x3x3 only) over the output box box6 = {d_lo, d_cnt, h_lo, h_cnt, w_lo, w_cnt} of a layer
+ * packed with the kh-shared flag (256): kh-shared M tiles over the largest multiple of 32 columns of the box, and 8-wide
+ * tiles over the rest (an 8-wide strip ending at w_lo + w_cnt that overlaps the main tiles) -- the launches
+ * oai_seg_forward makes for dc2 and dc1.  Voxels outside the box may be written, always with their full-layer values
+ * (whole M tiles, clamped into the grid); slices outside the d range are left untouched. */
+OAI_API int oai_conv3d_igemm_box(const void* src0, int c0, const void* src1, int c1, int in_split, const void* in_lo8,
+                                 int NT, int D, int H, int W, const void* wpack, size_t wpack_bytes, const float* bias,
+                                 int cout, int relu, int ab_format, int terms, void* out, int out_split, void* out_lo8,
+                                 int flags, const int* box6, void* stream);
 
 /* fp16 saturation guard: how many epilogue threads of the conv kernel (on the current device, since the last reset) saw
  * an activation outside the fp16 range (|x| > 65504, or NaN) before rounding it.  Non-zero means the 16-bit tensors hold

@@ -8,6 +8,7 @@
 #include <cuda_fp16.h>
 #include <cuda_fp8.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <vector>
@@ -85,9 +86,23 @@ int build_chunks(const ConvSpec& s, Plan* pl) {
   return 0;
 }
 
-// tw: M tile width of a kh-shared layer (8, 16 or 32); the packed weights do not depend on it
-int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0, int tw = 32) {
+// kh-shared tile width over an h_cnt x w_cnt box: the fewest M tiles, the widest on a tie (dc1's 96 x 96 box: 72 tiles
+// at every width; 32 x 4 and 8 x 16 tiles measured the same, 7.98 / 7.90 ms, though the 8-wide box is 25 % fewer bytes)
+int kh_tile_width(int H, int W, int h_cnt, int w_cnt) {
+  int tw = 32, ntile = 0;
+  for (int t = 32; t >= 8; t /= 2) {
+    if (t > W || 128 / t > H) continue;
+    const int n = ((w_cnt + t - 1) / t) * ((h_cnt + 128 / t - 1) / (128 / t));
+    if (ntile == 0 || n < ntile) { ntile = n; tw = t; }
+  }
+  return tw;
+}
+
+// tw: M tile width of a kh-shared layer (8, 16 or 32; 0: the width a launch over the whole grid takes); the packed
+// weights do not depend on it
+int make_plan(const ConvSpec& s, Plan* pl, int d_cnt = 0, int tw = 0) {
   const int D = s.D, H = s.H, W = s.W, c0 = s.c0, c1 = s.c1, cout = s.cout, pointwise = s.kind, flags = s.flags;
+  if (tw == 0) tw = kh_tile_width(H, W, H, W);
   OAI_REQUIRE(D > 0 && H > 0 && W > 0 && c0 > 0 && c1 >= 0 && cout > 0, "conv plan: bad dims");
   OAI_REQUIRE(c0 % 8 == 0 && c1 % 8 == 0, "conv plan: channel counts must be multiples of 8 (got %d,%d)", c0, c1);
   OAI_REQUIRE(s.terms >= 1 && s.terms <= 7,
@@ -453,17 +468,8 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
     OAI_REQUIRE(kh_shared, "conv: a w range needs a layer packed for kh-shared mode");
     OAI_REQUIRE(w_lo >= 0 && w_cnt >= 1 && w_lo + w_cnt <= W, "conv: w range [%d,+%d) outside W=%d", w_lo, w_cnt, W);
   }
-  // kh-shared tile width: the fewest M tiles over the box, the widest on a tie (dc1's 96 x 96 box: 72 tiles at every
-  // width; 32 x 4 and 8 x 16 tiles measured the same, 7.98 / 7.90 ms, though the 8-wide box is 25 % fewer bytes)
-  int tw = 32, ntile = 0;
-  if (kh_shared)
-    for (int t = 32; t >= 8; t /= 2) {
-      if (t > W || 128 / t > H) continue;
-      const int n = ((w_cnt + t - 1) / t) * ((h_cnt + 128 / t - 1) / (128 / t));
-      if (ntile == 0 || n < ntile) { ntile = n; tw = t; }
-    }
   Plan pl;
-  if (make_plan(s, &pl, d_cnt, tw)) return 1;
+  if (make_plan(s, &pl, d_cnt, kh_shared ? kh_tile_width(H, W, h_cnt, w_cnt) : 32)) return 1;
   int tile_h_lo = h_lo, nph = (h_cnt + pl.TH - 1) / pl.TH, npw = (w_cnt + pl.TW - 1) / pl.TW;
   if (!kh_shared) {   // whole M-tile rows of whole-row (or whole-grid-aligned) tiles
     tile_h_lo = h_lo / pl.TH * pl.TH;
@@ -559,6 +565,19 @@ int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st) {
   return check_cuda(e, "conv_igemm launch");
 }
 
+int conv_run_w_box(const ConvSpec& s, ConvLaunch a, int w_lo, int w_hi, cudaStream_t st) {
+  const int w_cnt = w_hi - w_lo + 1, main = w_cnt / 32 * 32, rest = w_cnt - main;
+  if (main) {
+    a.w_lo = w_lo; a.w_cnt = main; a.flop_share = static_cast<double>(main) / w_cnt;
+    if (int rc = conv_run(s, a, st)) return rc;
+  }
+  if (!rest) return 0;
+  a.w_cnt = std::min((rest + 7) / 8 * 8, w_cnt);
+  a.w_lo = w_hi + 1 - a.w_cnt;
+  a.flop_share = static_cast<double>(rest) / w_cnt;   // the layer's algorithmic MACs are booked once
+  return conv_run(s, a, st);
+}
+
 }  // namespace oai
 
 using namespace oai;
@@ -618,12 +637,15 @@ extern "C" int oai_pack_conv_weights_ex(const float* w, int cout, int c0, int c1
 static int conv_common(const void* src0, int c0, const void* src1, int c1, int NT, int D, int H, int W,
                        const void* wpack, size_t wpack_bytes, const float* bias, int cout, int pointwise, int relu,
                        int ab_format, void* out, long long obase, long long osN, long long osD, long long osH,
-                       long long osW, int flags, const HeadFuse* head, const int* region, void* stream) {
+                       long long osW, int flags, const HeadFuse* head, const int* region, void* stream,
+                       const int* w_range = nullptr) {
   ConvLaunch a;
   a.src0 = src0; a.src1 = src1; a.NT = NT; a.wpack = wpack; a.wpack_bytes = wpack_bytes; a.bias = bias; a.relu = relu;
   a.out = out; a.obase = obase; a.osN = osN; a.osD = osD; a.osH = osH; a.osW = osW; a.out_split = 0; a.out_lo_off = 0;
   a.region = region; a.head = head;
-  return conv_run(spec_of(D, H, W, c0, c1, cout, pointwise, ab_format, flags), a, static_cast<cudaStream_t>(stream));
+  const ConvSpec s = spec_of(D, H, W, c0, c1, cout, pointwise, ab_format, flags);
+  if (w_range) return conv_run_w_box(s, a, w_range[0], w_range[1], static_cast<cudaStream_t>(stream));
+  return conv_run(s, a, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int oai_conv3d_igemm(const void* src0, int c0, const void* src1, int c1, int NT, int D, int H, int W,
@@ -657,11 +679,10 @@ extern "C" int oai_conv3d_igemm_ex(const void* src0, int c0, const void* src1, i
 
 // ... with e4m3 lo planes: in_lo8 is the lo plane of the source terms 6 / 7 read (one byte per channel and voxel),
 // out_lo8 (optional, with out_split = 0) receives the output's lo plane.
-extern "C" int oai_conv3d_igemm_lo8(const void* src0, int c0, const void* src1, int c1, int in_split,
-                                    const void* in_lo8, int NT, int D, int H, int W, const void* wpack,
-                                    size_t wpack_bytes, const float* bias, int cout, int pointwise, int relu,
-                                    int ab_format, int terms, void* out, int out_split, void* out_lo8, int flags,
-                                    const int* region, void* stream) {
+static int conv_lo8_common(const void* src0, int c0, const void* src1, int c1, int in_split, const void* in_lo8, int NT,
+                           int D, int H, int W, const void* wpack, size_t wpack_bytes, const float* bias, int cout,
+                           int pointwise, int relu, int ab_format, int terms, void* out, int out_split, void* out_lo8,
+                           int flags, const int* region, const int* w_range, void* stream) {
   OAI_REQUIRE(out != nullptr, "conv: null output");
   OAI_REQUIRE(pointwise == 0 || pointwise == 1 || pointwise == 2, "conv: pointwise=%d", pointwise);
   ConvSpec s = spec_of(D, H, W, c0, c1, cout, pointwise, ab_format, flags);
@@ -678,7 +699,33 @@ extern "C" int oai_conv3d_igemm_lo8(const void* src0, int c0, const void* src1, 
   } else {
     a.osN = 1ll * D * H * W * cp; a.osD = 1ll * H * W * cp; a.osH = 1ll * W * cp; a.osW = cp;
   }
+  if (w_range) return conv_run_w_box(s, a, w_range[0], w_range[1], static_cast<cudaStream_t>(stream));
   return conv_run(s, a, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int oai_conv3d_igemm_lo8(const void* src0, int c0, const void* src1, int c1, int in_split,
+                                    const void* in_lo8, int NT, int D, int H, int W, const void* wpack,
+                                    size_t wpack_bytes, const float* bias, int cout, int pointwise, int relu,
+                                    int ab_format, int terms, void* out, int out_split, void* out_lo8, int flags,
+                                    const int* region, void* stream) {
+  return conv_lo8_common(src0, c0, src1, c1, in_split, in_lo8, NT, D, H, W, wpack, wpack_bytes, bias, cout, pointwise,
+                         relu, ab_format, terms, out, out_split, out_lo8, flags, region, nullptr, stream);
+}
+
+extern "C" int oai_conv3d_igemm_box(const void* src0, int c0, const void* src1, int c1, int in_split,
+                                    const void* in_lo8, int NT, int D, int H, int W, const void* wpack,
+                                    size_t wpack_bytes, const float* bias, int cout, int relu, int ab_format, int terms,
+                                    void* out, int out_split, void* out_lo8, int flags, const int* box6, void* stream) {
+  OAI_REQUIRE(box6 != nullptr, "conv box: null box");
+  OAI_REQUIRE(flags & kConvFlagKhShared, "conv box: the layer must be packed and run kh-shared (flag %d)",
+              kConvFlagKhShared);
+  OAI_REQUIRE(box6[0] >= 0 && box6[1] >= 1 && box6[0] + box6[1] <= D && box6[2] >= 0 && box6[3] >= 1 &&
+                  box6[2] + box6[3] <= H && box6[4] >= 0 && box6[5] >= 1 && box6[4] + box6[5] <= W,
+              "conv box: [%d,+%d)x[%d,+%d)x[%d,+%d) outside the %dx%dx%d grid", box6[0], box6[1], box6[2], box6[3],
+              box6[4], box6[5], D, H, W);
+  const int w_range[2] = {box6[4], box6[4] + box6[5] - 1};
+  return conv_lo8_common(src0, c0, src1, c1, in_split, in_lo8, NT, D, H, W, wpack, wpack_bytes, bias, cout, 0, relu,
+                         ab_format, terms, out, out_split, out_lo8, flags, box6, w_range, stream);
 }
 
 extern "C" int oai_conv3d_igemm_head(const void* src0, int c0, const void* src1, int c1, int NT, int D, int H, int W,
@@ -692,8 +739,10 @@ extern "C" int oai_conv3d_igemm_head(const void* src0, int c0, const void* src1,
   // only the tile interior is ever written, so only the interior rows are computed
   const int region[4] = {geom[6], geom[3], geom[7], geom[4]};
   HeadFuse hd = make_head_fuse(ncls, head_w, head_b, out, vol_dims, geom, tile0, crop_zyx, out_mode);
+  // a kh-shared layer computes only the interior columns too, as oai_seg_forward's last step does
+  const int w_range[2] = {geom[8], geom[8] + geom[5] - 1};
   return conv_common(src0, c0, src1, c1, NT, D, H, W, wpack, wpack_bytes, bias, 64, 0, 1, ab_format, nullptr, 0, 0, 0,
-                     0, 0, flags, &hd, region, stream);
+                     0, 0, flags, &hd, region, stream, (flags & kConvFlagKhShared) ? w_range : nullptr);
 }
 
 extern "C" int oai_conv_overflow_count(long long* count, int reset, void* stream) {

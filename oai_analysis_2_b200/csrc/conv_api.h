@@ -49,6 +49,10 @@ struct ConvLaunch {
 size_t conv_wpack_bytes(const ConvSpec& s);
 int conv_pack_weights(const ConvSpec& s, const float* w, void* dst, size_t dst_bytes);
 int conv_run(const ConvSpec& s, const ConvLaunch& a, cudaStream_t st);
+// A kh-shared launch (kConvFlagKhShared) over the w range [w_lo, w_hi] of a.region: 32-wide M tiles over the largest
+// multiple of 32 columns, and a second launch of 8-wide tiles over the last columns when the width is not a multiple of
+// 32 (dc2: 98 = 96 + 2, the strip covers the last 8 and overlaps the main tiles, which write the same values there).
+int conv_run_w_box(const ConvSpec& s, ConvLaunch a, int w_lo, int w_hi, cudaStream_t st);
 
 inline HeadFuse make_head_fuse(int ncls, const float* head_w, const float* head_b, float* out, const int* vol_dims,
                                const int* geom, int tile0, const int* crop_zyx, int out_mode) {

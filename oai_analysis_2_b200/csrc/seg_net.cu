@@ -459,21 +459,6 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
   const int crop_zyx[3] = {h->cfg.overlap_xyz[2], h->cfg.overlap_xyz[0], h->cfg.overlap_xyz[1]};
   const int fmt = h->cfg.ab_format;
 
-  // a kh-shared launch over the w range [w_lo, w_hi]: 32-wide M tiles over the largest multiple of 32 columns, and a
-  // second launch of 8-wide tiles over the last columns when the width is not a multiple of 32 (dc2: 98 = 96 + 2, the
-  // strip covers the last 8 and overlaps the main tiles, which write the same values there)
-  auto conv_w_box = [&](const ConvSpec& s, ConvLaunch a, int w_lo, int w_hi) -> int {
-    const int w_cnt = w_hi - w_lo + 1, main = w_cnt / 32 * 32, rest = w_cnt - main;
-    if (main) {
-      a.w_lo = w_lo; a.w_cnt = main; a.flop_share = static_cast<double>(main) / w_cnt;
-      if (int rc = conv_run(s, a, st)) return rc;
-    }
-    if (!rest) return 0;
-    a.w_cnt = std::min((rest + 7) / 8 * 8, w_cnt);
-    a.w_lo = w_hi + 1 - a.w_cnt;
-    a.flop_share = static_cast<double>(rest) / w_cnt;   // the layer's algorithmic MACs are booked once
-    return conv_run(s, a, st);
-  };
   auto conv = [&](int l, int NT, int t0, int t1, int tout) -> int {
     const LayerDef& L = kLayers[l];
     const PackedLayer& P = h->layers[l];
@@ -504,7 +489,7 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
       a.region = region;
     }
     a.head = nullptr;
-    if (a.region && (s.flags & kConvFlagKhShared)) return conv_w_box(s, a, h->region[l].lo[2], h->region[l].hi[2]);
+    if (a.region && (s.flags & kConvFlagKhShared)) return conv_run_w_box(s, a, h->region[l].lo[2], h->region[l].hi[2], st);
     return conv_run(s, a, st);
   };
   auto pool = [&](int i, int NT) -> int {
@@ -557,7 +542,7 @@ extern "C" int oai_seg_forward(oai_seg_t h, const float* vol, const int* vol_dim
     a.src0 = buf(T_D2); a.src1 = nullptr; a.NT = NT; a.wpack = P.w; a.wpack_bytes = P.w_bytes; a.bias = P.bias;
     a.relu = 1; a.out = nullptr; a.obase = a.osN = a.osD = a.osH = a.osW = 0; a.out_split = 0; a.out_lo_off = 0;
     a.region = region; a.head = &hd; a.src_lo8 = lo8buf(T_D2);
-    rc = (s.flags & kConvFlagKhShared) ? conv_w_box(s, a, geom[8], geom[8] + geom[5] - 1) : conv_run(s, a, st);
+    rc = (s.flags & kConvFlagKhShared) ? conv_run_w_box(s, a, geom[8], geom[8] + geom[5] - 1, st) : conv_run(s, a, st);
   }
   nvtxRangePop();
   return rc;

@@ -244,23 +244,46 @@ def pack_conv_weights_ex(w, c0, c1, D, H, W, pointwise=0, terms=1, ab_format=0, 
 
 
 def conv3d_igemm_ex(src0, src1, wpack, bias, cout, c0, c1=0, pointwise=0, relu=True, ab_format=0, terms=1,
-                    in_split=False, out_split=False, region=None, flags=0, in_lo8=None, out_lo8=False):
+                    in_split=False, out_split=False, region=None, flags=0, in_lo8=None, out_lo8=False, out=None):
     """Split-precision form of conv3d_igemm: src* are [NT,D,H,W,C] (or [.., 2C] = [hi | lo] when in_split).
     terms 6 / 7: in_lo8 is the uint8 e4m3 lo plane of the split source (split_lo8); out_lo8: also return the output's
-    lo plane, (out, lo8)."""
+    lo plane, (out, lo8).  out (optional): the dense output tensor to write into; out_lo8 may then be a uint8 tensor of
+    the same shape to receive the lo plane.  Voxels a region launch does not compute keep what these tensors held."""
     NT, D, H, W, _ = src0.shape
     assert src0.is_contiguous() and (src1 is None or src1.is_contiguous())
     assert in_lo8 is None or (in_lo8.dtype == torch.uint8 and in_lo8.is_contiguous())
     up = 2 if pointwise == 2 else 1
-    out = torch.empty((NT, up * D, up * H, up * W, cout * (2 if out_split else 1)), dtype=_DT16[ab_format],
-                      device=src0.device)
-    lo8 = torch.empty(out.shape, dtype=torch.uint8, device=src0.device) if out_lo8 else None
+    shape = (NT, up * D, up * H, up * W, cout * (2 if out_split else 1))
+    if out is None:
+        out = torch.empty(shape, dtype=_DT16[ab_format], device=src0.device)
+    assert tuple(out.shape) == shape and out.dtype == _DT16[ab_format] and out.is_contiguous(), "conv: bad out tensor"
+    if isinstance(out_lo8, torch.Tensor):
+        lo8 = out_lo8
+        assert tuple(lo8.shape) == tuple(out.shape) and lo8.dtype == torch.uint8 and lo8.is_contiguous()
+    else:
+        lo8 = torch.empty(out.shape, dtype=torch.uint8, device=src0.device) if out_lo8 else None
     reg = None if region is None else np.asarray(region, dtype=np.int32)
     check(lib.oai_conv3d_igemm_lo8(ptr(src0), c0, ptr(src1), c1, int(in_split), ptr(in_lo8), NT, D, H, W, ptr(wpack),
                                    c_size(wpack.numel()), ptr(bias), cout, int(pointwise), int(relu), ab_format,
                                    int(terms), ptr(out), int(out_split), ptr(lo8), flags, ptr(reg), stream_ptr()),
           "conv3d_igemm_ex")
-    return (out, lo8) if out_lo8 else out
+    return (out, lo8) if lo8 is not None else out
+
+
+def conv3d_igemm_box(src0, src1, wpack, bias, cout, c0, c1, box6, relu=True, ab_format=0, terms=1, in_split=False,
+                     out_split=False, flags=0, in_lo8=None, out=None, out_lo8=None):
+    """oai_conv3d_igemm_box: a kh-shared 3x3x3 layer over box6 = (d_lo, d_cnt, h_lo, h_cnt, w_lo, w_cnt), the launches
+    the segmenter makes for dc2 / dc1.  Same tensors as conv3d_igemm_ex; out / out_lo8 must be given (the box writes
+    only part of them)."""
+    NT, D, H, W, _ = src0.shape
+    assert src0.is_contiguous() and (src1 is None or src1.is_contiguous()) and out is not None and out.is_contiguous()
+    assert tuple(out.shape) == (NT, D, H, W, cout * (2 if out_split else 1)) and out.dtype == _DT16[ab_format]
+    assert out_lo8 is None or (out_lo8.shape == out.shape and out_lo8.dtype == torch.uint8 and out_lo8.is_contiguous())
+    box = np.asarray(box6, dtype=np.int32)
+    check(lib.oai_conv3d_igemm_box(ptr(src0), c0, ptr(src1), c1, int(in_split), ptr(in_lo8), NT, D, H, W, ptr(wpack),
+                                   c_size(wpack.numel()), ptr(bias), cout, int(relu), ab_format, int(terms), ptr(out),
+                                   int(out_split), ptr(out_lo8), flags, ptr(box), stream_ptr()), "conv3d_igemm_box")
+    return out
 
 
 def seg_head(act, w, b, out, geom, tile0, crop_zyx, out_mode=0, ab_format=0):
